@@ -3,7 +3,7 @@
 megapixels per second at 1/2/4/8 B200, fraction of the tensor roofline, PSNR / bpp parity).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
-                    [--workload wsi|patches|train]
+                    [--workload wsi|patches|train] [--dump-outputs DIR]
 
 Default workload ``wsi`` (BASELINE.json configs 3/4): a synthetic tissue-like whole-slide image
 of 512 x 512 chunks, net A (3->128->128->48, level 3, LeakyReLU, random-init weights), sharded
@@ -25,6 +25,14 @@ the CPU oracle), ``roofline`` of the dominant kernel timed alone, ``device_resid
 (the config-2 CUDA-graph replay of round 1, no entropy coding), ``cpu_baseline`` (the oracle on
 this box's cores, bounded sample).  ``--workload patches`` is the round-1 bench (config 2) in
 full; ``--workload train`` is the rate-distortion training step (config 5).
+
+``--dump-outputs DIR`` (workload ``wsi``) writes what the last timed step of each region handed
+its caller, so that two builds can be compared output for output on identical seeded inputs:
+``DUMP_CHUNKS`` chunks of the reconstruction picked by a fixed seed (float32, N x 512 x 512 x 3,
+uint8 values) from the e2e and the device-resident run, the stored bytes of each, the stored
+chunk files (16-byte header + rANS stream, byte values as float32, back to back, with their
+lengths) of the same chunks from the last step of the raw-chunk-file e2e variant, which keeps its
+store, and the picked chunks' (row, column) indices (float64).
 """
 import argparse
 import json
@@ -44,6 +52,7 @@ BATCH, SIZE = 128, 256                  # config 2
 PS, TILES, GX = 512, 8192, 64           # configs 3/4: chunk size, chunks per GPU, chunks per row
 FLOPS_PER_PX = {'A': 136746, 'A_res': 321876, 'B': 367236, 'M': 738}   # SURVEY.md 8d
 METRIC = 'wsi_encode_decode_megapixels_per_sec'
+DUMP_CHUNKS = 8                         # 2 x 8 float32 chunks of 512 x 512 x 3 + streams: ~55 MB of dump
 ARCH_TEXT = {'A': 'net A (3->128->128->48 L3 LeakyReLU)', 'A_res': 'net A+res',
              'B': 'net B (192 latent channels, L4, residual)'}
 
@@ -427,6 +436,8 @@ def run_wsi(args):
     # prologue.  Every call, copy and file operation of the K steps lies inside the timed region;
     # `e2e.one_step_at_a_time` is the same measured with the calls strictly one after the other.
     my_chunks = [(i, j, 0) for i in range(rank * rows_per_rank, (rank + 1) * rows_per_rank) for j in range(GX)]
+    dump = {} if args.dump_outputs and rank == 0 else None
+    dump_yx = [my_chunks[k][:2] for k in sorted(np.random.default_rng(0).choice(T, DUMP_CHUNKS, replace=False))]
     cleaner = ThreadPoolExecutor(max_workers=1)
     jobs = SlideJobs(c.local)
     state = dict(step=0, dec={}, clean={})
@@ -508,6 +519,10 @@ def run_wsi(args):
                 state.update(step=state['step'] + 2, dec={}, clean={})
         if args.e2e_in_flight == 1:
             done, e2e_ms, wall = timed(lambda: [run(1)[0] for _ in range(args.steps)])
+        if dump is not None:      # taken now: the variants below write the reconstruction again
+            dump['e2e_reconstruction'] = np.stack([recon[i * PS:(i + 1) * PS, j * PS:(j + 1) * PS]
+                                                   for i, j in dump_yx]).astype(np.float32)
+            dump['e2e_stored_bytes'] = np.array([done[-1][0]['bytes']], np.float64)
         for cs, ds in done:
             for k, v in (('compress_s', cs['seconds']), ('decompress_s', ds['seconds'])):
                 phases[k] = phases.get(k, 0.0) + v
@@ -529,6 +544,10 @@ def run_wsi(args):
         cs, ds = files[-1]
         e2e_files_value = world * px_step * 2 / (files_ms / 1e3) / 1e6
         stored = DirArray(os.path.join(cs['store'], '0/0'), mode='r')       # the last step's store is kept
+        if dump is not None:      # what compress_image stored for the sampled chunks: header + rANS stream
+            streams = [np.frombuffer(stored.read_encoded((i, j, 0)), np.uint8) for i, j in dump_yx]
+            dump['e2e_chunk_streams'] = np.concatenate(streams).astype(np.float32)
+            dump['e2e_chunk_stream_bytes'] = np.array([s.size for s in streams], np.float64)
         comp_bytes_rank = cs['bytes']
 
         # ---- value: the same codec, everything resident in HBM ----
@@ -550,7 +569,7 @@ def run_wsi(args):
         t_begin = time.time()
         for s, e in ev:
             s.record()
-            _slide.device_roundtrip(tc, x_dev, out_dev, args.coder_tiles)
+            stored_bytes = _slide.device_roundtrip(tc, x_dev, out_dev, args.coder_tiles)
             e.record()
         c.barrier()
         clk.window(t_begin, time.time())
@@ -558,6 +577,10 @@ def run_wsi(args):
                     (tc.replays_dec - replays0[1]) * tc.launches_dec)
         total_ms = c.max_over_ranks(sum(s.elapsed_time(e) for s, e in ev))
         value = world * px_step * args.steps / (total_ms / 1e3) / 1e6
+        if dump is not None:
+            k = [(i - rank * rows_per_rank) * GX + j for i, j in dump_yx]
+            dump['device_reconstruction'] = out_dev[k].cpu().numpy().astype(np.float32)
+            dump['device_stored_bytes'] = np.array([stored_bytes], np.float64)
     clocks = clk.summary()
     clk.window(*clk_e2e_window)
     clocks_e2e = clk.summary()
@@ -698,6 +721,11 @@ def run_wsi(args):
         'parity': parity, 'device_resident_patches': sub,
         'roofline': roof, 'cpu_baseline': cpu,
     }
+    if dump is not None:
+        dump['chunks'] = np.array(dump_yx, np.float64)
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in dump.items():
+            np.save(os.path.join(args.dump_outputs, name + '.npy'), a)
     print(json.dumps(line))
     pin.close()
     pin_r.close()
@@ -837,7 +865,11 @@ def main():
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--no-graph', action='store_true',
                     help='issue every kernel from Python instead of replaying CUDA graphs')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write the outputs of the last timed step as DIR/<name>.npy (workload wsi)')
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != 'ours' or args.workload != 'wsi'):
+        ap.error('--dump-outputs writes the outputs of --workload wsi with --impl ours')
     if any(k in os.environ for k in ('CUDA_INJECTION64_PATH', 'NV_COMPUTE_PROFILER_PERFWORKS_DIR',
                                      'NV_NSIGHT_INJECTION_PORT_BASE')) and not args.no_graph:
         # ncu --set full cannot replay the tensor-map kernels as graph nodes (profiles/README.md)
