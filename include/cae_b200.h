@@ -399,6 +399,16 @@ int cae_tiles_download_u8_banded(const uint8_t *src, int n, int ps, int c,
                                  const int32_t *tile_yx /*HOST*/, uint8_t *dst /*HOST*/, int64_t H,
                                  int64_t W, uint8_t *scratch, void *stream);
 
+/* Region reads: windows cut out of one batch of decoded tiles, on the device.  `tiles`: tile-major
+ * n_tiles x ps x ps x c; `out`: n_boxes x box_h x box_w x c.  Piece i = pieces[8i .. 8i+7] =
+ * {k, b, sy, sx, dy, dx, h, w}: rows [sy, sy+h) x columns [sx, sx+w) of tile k go to (dy, dx) of
+ * box b; k = -1 writes zeros instead (the fill value of a chunk whose file is missing).  Every
+ * piece is checked on the host before the table is copied to `pieces_dev` (DEVICE, m x 8 int32,
+ * 16-byte aligned) on `stream`; one launch copies them all.                                    */
+int cae_tiles_crop_u8(const uint8_t *tiles, int n_tiles, int ps, int c,
+                      const int32_t *pieces /*HOST, m x 8*/, int m, int32_t *pieces_dev /*m x 8*/,
+                      uint8_t *out, int n_boxes, int box_h, int box_w, void *stream);
+
 /* ---- evaluation sums on the device (SURVEY.md 8f-4) ------------------------------------------ */
 /* sse[i] += sum over the per_image uint8 values of image i of (a - b)^2: the numerator of
  * compute_rmse / compute_psnr (src/test_cae.py:57-63, computed there on the host after a full
