@@ -146,12 +146,13 @@ extern "C" int cae_tiles_upload_u8_banded(const uint8_t *src, int64_t H, int64_t
 }
 
 // ---------------------------------------------------------------------------------------------
-// Region reads (region.py): windows cut out of a batch of decoded tiles.  A piece
-// {k, b, sy, sx, dy, dx, h, w} copies rows [sy, sy + h) x columns [sx, sx + w) of tile k to
-// (dy, dx) of box b; k = -1 writes zeros (zarr's fill value for a chunk whose file is missing).
-// HBM bound.  Block (p, q) copies rows [q * rows, (q + 1) * rows) of piece p in the widest unit
-// that the piece's source rows, destination rows and row length all allow (16, 4 or 1 bytes):
-// with c = 3 and windows at arbitrary offsets the byte loop is the common case.
+// Region reads and writes (region.py).  A piece {k, b, sy, sx, dy, dx, h, w} pairs rows
+// [sy, sy + h) x columns [sx, sx + w) of tile k with rows [dy, dy + h) x columns [dx, dx + w) of
+// box b.  cae_tiles_crop_u8 copies tile -> box (k = -1 writes zeros: zarr's fill value for a chunk
+// whose file is missing); cae_tiles_paste_u8 copies box -> tile (b = -1 writes zeros: the padding
+// of edge chunks).  HBM bound.  Block (p, q) copies rows [q * rows, (q + 1) * rows) of piece p in
+// the widest unit that the piece's source rows, destination rows and row length all allow (16, 4
+// or 1 bytes): with c = 3 and windows at arbitrary offsets the byte loop is the common case.
 namespace {
 constexpr int kCropThreads = 256;
 
@@ -168,6 +169,16 @@ __device__ __forceinline__ void crop_rows(const uint8_t *src, size_t src_pitch, 
   }
 }
 
+// `rows` rows of `row_bytes` from src (nullptr: zeros) to dst in the widest unit that fits
+__device__ __forceinline__ void copy_rows(const uint8_t *src, size_t src_pitch, uint8_t *dst,
+                                          size_t dst_pitch, int rows, int row_bytes) {
+  const uintptr_t bits = reinterpret_cast<uintptr_t>(dst) | dst_pitch | (uintptr_t)row_bytes |
+                         (src ? reinterpret_cast<uintptr_t>(src) | src_pitch : 0);
+  if ((bits & 15) == 0) crop_rows<uint4>(src, src_pitch, dst, dst_pitch, rows, row_bytes);
+  else if ((bits & 3) == 0) crop_rows<uint32_t>(src, src_pitch, dst, dst_pitch, rows, row_bytes);
+  else crop_rows<uint8_t>(src, src_pitch, dst, dst_pitch, rows, row_bytes);
+}
+
 __global__ void __launch_bounds__(kCropThreads) tiles_crop_u8_kernel(
     const uint8_t *__restrict__ tiles, int ps, int c, const int4 *__restrict__ pieces,
     uint8_t *__restrict__ out, int box_h, int box_w, int rows_per_block) {
@@ -175,17 +186,58 @@ __global__ void __launch_bounds__(kCropThreads) tiles_crop_u8_kernel(
   const int k = p0.x, b = p0.y, sy = p0.z, sx = p0.w, dy = p1.x, dx = p1.y, h = p1.z, w = p1.w;
   const int r0 = blockIdx.y * rows_per_block;
   if (r0 >= h) return;
-  const int rows = min(rows_per_block, h - r0);
-  const size_t src_pitch = (size_t)ps * c, dst_pitch = (size_t)box_w * c;
-  const int row_bytes = w * c;
   const uint8_t *src = k < 0 ? nullptr
                              : tiles + (((size_t)k * ps + sy + r0) * ps + sx) * c;
   uint8_t *dst = out + (((size_t)b * box_h + dy + r0) * box_w + dx) * c;
-  const uintptr_t bits = reinterpret_cast<uintptr_t>(dst) | dst_pitch | (uintptr_t)row_bytes |
-                         (src ? reinterpret_cast<uintptr_t>(src) | src_pitch : 0);
-  if ((bits & 15) == 0) crop_rows<uint4>(src, src_pitch, dst, dst_pitch, rows, row_bytes);
-  else if ((bits & 3) == 0) crop_rows<uint32_t>(src, src_pitch, dst, dst_pitch, rows, row_bytes);
-  else crop_rows<uint8_t>(src, src_pitch, dst, dst_pitch, rows, row_bytes);
+  copy_rows(src, (size_t)ps * c, dst, (size_t)box_w * c, min(rows_per_block, h - r0), w * c);
+}
+
+__global__ void __launch_bounds__(kCropThreads) tiles_paste_u8_kernel(
+    uint8_t *__restrict__ tiles, int ps, int c, const int4 *__restrict__ pieces,
+    const uint8_t *__restrict__ boxes, int box_h, int box_w, int rows_per_block) {
+  const int4 p0 = pieces[2 * blockIdx.x], p1 = pieces[2 * blockIdx.x + 1];
+  const int k = p0.x, b = p0.y, sy = p0.z, sx = p0.w, dy = p1.x, dx = p1.y, h = p1.z, w = p1.w;
+  const int r0 = blockIdx.y * rows_per_block;
+  if (r0 >= h) return;
+  const uint8_t *src = b < 0 ? nullptr
+                             : boxes + (((size_t)b * box_h + dy + r0) * box_w + dx) * c;
+  uint8_t *dst = tiles + (((size_t)k * ps + sy + r0) * ps + sx) * c;
+  copy_rows(src, (size_t)box_w * c, dst, (size_t)ps * c, min(rows_per_block, h - r0), w * c);
+}
+
+// Host side of both: every piece is checked before anything is copied or launched (k >= tile_min,
+// b >= box_min; a piece lies inside its tile, and inside its box unless b = -1), then the table
+// goes up to pieces_dev on the stream and the grid is sized.
+int check_pieces(const char *fn, const int32_t *pieces, int m, int n_tiles, int tile_min,
+                 int n_boxes, int box_min, int ps, int c, int box_h, int box_w, dim3 *grid,
+                 int *rows_per_block) {
+  CAE_CHECK((int64_t)ps * ps * c <= INT32_MAX && (int64_t)box_w * c <= INT32_MAX, 2,
+            "%s: tile or box row too large", fn);
+  int max_h = 0, max_row = 0;
+  for (int i = 0; i < m; ++i) {
+    const int32_t *p = pieces + 8 * (size_t)i;
+    const int k = p[0], b = p[1], sy = p[2], sx = p[3], dy = p[4], dx = p[5], h = p[6], w = p[7];
+    CAE_CHECK(k >= tile_min && k < n_tiles, 2, "%s: piece %d names tile %d of %d", fn, i, k,
+              n_tiles);
+    CAE_CHECK(b >= box_min && b < n_boxes, 2, "%s: piece %d names box %d of %d", fn, i, b,
+              n_boxes);
+    CAE_CHECK(h > 0 && w > 0 && sy >= 0 && sx >= 0 && sy <= ps - h && sx <= ps - w, 2,
+              "%s: piece %d (rows %d+%d, columns %d+%d) lies outside its %d^2 tile",
+              fn, i, sy, h, sx, w, ps);
+    CAE_CHECK(b < 0 || (dy >= 0 && dx >= 0 && dy <= box_h - h && dx <= box_w - w), 2,
+              "%s: piece %d (rows %d+%d, columns %d+%d) lies outside its %d x %d box",
+              fn, i, dy, h, dx, w, box_h, box_w);
+    max_h = h > max_h ? h : max_h;
+    max_row = w * c > max_row ? w * c : max_row;
+  }
+  // ~8 KB per block: enough work to hide the piece lookup, enough blocks for small requests
+  int rows = 8192 / max_row;
+  rows = rows < 1 ? 1 : rows > 64 ? 64 : rows;
+  const int grid_y = (max_h + rows - 1) / rows;
+  CAE_CHECK(grid_y <= 65535, 2, "%s: pieces of %d rows are too tall", fn, max_h);
+  *grid = dim3((unsigned)m, (unsigned)grid_y);
+  *rows_per_block = rows;
+  return 0;
 }
 }  // namespace
 
@@ -198,35 +250,41 @@ extern "C" int cae_tiles_crop_u8(const uint8_t *tiles, int n_tiles, int ps, int 
   CAE_CHECK(pieces && pieces_dev && out && (tiles || n_tiles == 0), 2,
             "cae_tiles_crop_u8: null pointer");
   CAE_CHECK((uintptr_t)pieces_dev % 16 == 0, 2, "cae_tiles_crop_u8: pieces_dev is not 16-byte aligned");
-  CAE_CHECK((int64_t)ps * ps * c <= INT32_MAX && (int64_t)box_w * c <= INT32_MAX, 2,
-            "cae_tiles_crop_u8: tile or box row too large");
-  int max_h = 0, max_row = 0;
-  for (int i = 0; i < m; ++i) {
-    const int32_t *p = pieces + 8 * (size_t)i;
-    const int k = p[0], b = p[1], sy = p[2], sx = p[3], dy = p[4], dx = p[5], h = p[6], w = p[7];
-    CAE_CHECK(k >= -1 && k < n_tiles, 2, "cae_tiles_crop_u8: piece %d names tile %d of %d", i, k,
-              n_tiles);
-    CAE_CHECK(b >= 0 && b < n_boxes, 2, "cae_tiles_crop_u8: piece %d names box %d of %d", i, b,
-              n_boxes);
-    CAE_CHECK(h > 0 && w > 0 && sy >= 0 && sx >= 0 && sy <= ps - h && sx <= ps - w, 2,
-              "cae_tiles_crop_u8: piece %d (rows %d+%d, columns %d+%d) lies outside its %d^2 tile",
-              i, sy, h, sx, w, ps);
-    CAE_CHECK(dy >= 0 && dx >= 0 && dy <= box_h - h && dx <= box_w - w, 2,
-              "cae_tiles_crop_u8: piece %d (rows %d+%d, columns %d+%d) lies outside its %d x %d box",
-              i, dy, h, dx, w, box_h, box_w);
-    max_h = h > max_h ? h : max_h;
-    max_row = w * c > max_row ? w * c : max_row;
-  }
-  // ~8 KB per block: enough work to hide the piece lookup, enough blocks for small requests
-  int rows = 8192 / max_row;
-  rows = rows < 1 ? 1 : rows > 64 ? 64 : rows;
-  const int grid_y = (max_h + rows - 1) / rows;
-  CAE_CHECK(grid_y <= 65535, 2, "cae_tiles_crop_u8: pieces of %d rows are too tall", max_h);
+  dim3 grid;
+  int rows;
+  if (int rc = check_pieces("cae_tiles_crop_u8", pieces, m, n_tiles, -1, n_boxes, 0, ps, c, box_h,
+                            box_w, &grid, &rows))
+    return rc;
   cudaStream_t st = (cudaStream_t)stream;
   CAE_CUDA(cudaMemcpyAsync(pieces_dev, pieces, sizeof(int32_t) * 8 * (size_t)m,
                            cudaMemcpyHostToDevice, st));
-  tiles_crop_u8_kernel<<<dim3((unsigned)m, (unsigned)grid_y), kCropThreads, 0, st>>>(
+  tiles_crop_u8_kernel<<<grid, kCropThreads, 0, st>>>(
       tiles, ps, c, reinterpret_cast<const int4 *>(pieces_dev), out, box_h, box_w, rows);
+  cae_count_launch();
+  CAE_CUDA(cudaGetLastError());
+  return 0;
+}
+
+extern "C" int cae_tiles_paste_u8(uint8_t *tiles, int n_tiles, int ps, int c,
+                                  const int32_t *pieces, int m, int32_t *pieces_dev,
+                                  const uint8_t *boxes, int n_boxes, int box_h, int box_w,
+                                  void *stream) {
+  CAE_CHECK(n_tiles >= 0 && ps > 0 && c > 0 && m >= 0 && n_boxes >= 0 && box_h > 0 && box_w > 0, 2,
+            "cae_tiles_paste_u8: bad argument");
+  if (m == 0) return 0;
+  CAE_CHECK(pieces && pieces_dev && tiles && (boxes || n_boxes == 0), 2,
+            "cae_tiles_paste_u8: null pointer");
+  CAE_CHECK((uintptr_t)pieces_dev % 16 == 0, 2, "cae_tiles_paste_u8: pieces_dev is not 16-byte aligned");
+  dim3 grid;
+  int rows;
+  if (int rc = check_pieces("cae_tiles_paste_u8", pieces, m, n_tiles, 0, n_boxes, -1, ps, c, box_h,
+                            box_w, &grid, &rows))
+    return rc;
+  cudaStream_t st = (cudaStream_t)stream;
+  CAE_CUDA(cudaMemcpyAsync(pieces_dev, pieces, sizeof(int32_t) * 8 * (size_t)m,
+                           cudaMemcpyHostToDevice, st));
+  tiles_paste_u8_kernel<<<grid, kCropThreads, 0, st>>>(
+      tiles, ps, c, reinterpret_cast<const int4 *>(pieces_dev), boxes, box_h, box_w, rows);
   cae_count_launch();
   CAE_CUDA(cudaGetLastError());
   return 0;

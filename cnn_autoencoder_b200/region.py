@@ -1,4 +1,4 @@
-"""Region reads from a compressed slide: decode only the chunks a window touches.
+"""Region reads from and writes to a compressed slide: code only the chunks a window touches.
 
 With the reference, a compressed slide is a zarr array whose ``'cae'`` codec is registered with
 numcodecs, so ``zarr.open(path)['0/0'][y0:y1, x0:x1]`` decodes the chunks under the window one
@@ -11,6 +11,15 @@ their streams in one device coder call (few streams go to the host coder on a th
 the synthesis transform over ``batch_tiles`` tiles at a time with the kernels of the whole-slide
 engine, and after every batch one launch of ``cae_tiles_crop_u8`` cuts the boxes' pieces out of
 the decoded tiles on the device.  The pixels are the ones ``decompress_image`` writes.
+
+Opened with ``mode='r+'`` (or made empty by ``create_slide``) it also writes, as zarr's
+assignment does: a read-modify-write per touched chunk.  ``write_plan`` adds to ``plan`` which
+chunks are covered whole (encoded without reading them) and the zero pieces of edge padding; the
+partly covered chunks are decoded as for a read, every batch of tiles is assembled on the device
+with one ``cae_tiles_paste_u8`` launch, encoded with the engine's kernels, entropy-coded per
+group and written as chunk files.  The padding of an edge chunk is always stored as zeros
+(``compress_image`` does the same; zarr would keep the decoded padding), so writing a slide in
+whole chunks gives ``compress_image``'s files byte for byte.
 """
 import os
 import struct
@@ -23,8 +32,8 @@ import torch
 from . import _autoencoders as AE
 from . import _cabi as C
 from . import _slide
-from ._entropy import decode_symbols
-from ._store import DirArray, _paths_blob, native_read
+from ._entropy import decode_symbols, encode_symbols
+from ._store import DirArray, _paths_blob, native_read, native_write
 
 
 def plan(shape, chunks, boxes, box_h, box_w):
@@ -75,6 +84,52 @@ def plan(shape, chunks, boxes, box_h, box_w):
     return chunk_yx, np.ascontiguousarray(pieces[order], dtype=np.int32)
 
 
+def check_disjoint(boxes, box_h, box_w):
+    """Raise ``ValueError`` if two of the ``box_h`` x ``box_w`` boxes at ``boxes`` (N x 2 top-left
+    (y, x)) share a pixel: a write of overlapping boxes would depend on their order."""
+    yx = np.asarray(boxes, dtype=np.int64).reshape(-1, 2)
+    order = np.lexsort((yx[:, 1], yx[:, 0]))
+    y, x = yx[order, 0], yx[order, 1]
+    # sorted by y: once no pair d apart is closer than box_h in y, no pair further apart is
+    for d in range(1, len(y)):
+        near = y[d:] - y[:-d] < box_h
+        if not near.any():
+            break
+        hit = near & (np.abs(x[d:] - x[:-d]) < box_w)
+        if hit.any():
+            i = int(np.argmax(hit))
+            a, b = sorted((int(order[i]), int(order[i + d])))
+            raise ValueError('boxes %d and %d overlap: a write would depend on their order' % (a, b))
+
+
+def write_plan(shape, chunks, boxes, box_h, box_w):
+    """What a write of the ``box_h`` x ``box_w`` boxes at ``boxes`` needs: ``plan`` plus, per
+    touched chunk, whether the boxes cover its whole in-array part, and the zero pieces of its
+    padding.
+
+    Returns ``(chunk_yx, pieces, full, fill)``: ``chunk_yx`` and ``pieces`` as ``plan`` returns
+    them; ``full``: bool K, the chunks whose in-array part is covered (they are encoded without
+    reading their old file); ``fill``: int32 F x 8 pieces ``{k, -1, sy, sx, 0, 0, h, w}`` covering
+    the part of every touched edge chunk beyond the array edge (stored as zeros).  Value and fill
+    pieces are pairwise disjoint.  Raises ``ValueError`` for overlapping boxes."""
+    chunk_yx, pieces = plan(shape, chunks, boxes, box_h, box_w)
+    check_disjoint(boxes, box_h, box_w)
+    H, W = int(shape[0]), int(shape[1])
+    cy, cx = int(chunks[0]), int(chunks[1])
+    ih = np.minimum(cy, H - chunk_yx[:, 0] * cy)          # in-array rows / columns of each chunk
+    iw = np.minimum(cx, W - chunk_yx[:, 1] * cx)
+    covered = np.bincount(pieces[:, 0], weights=pieces[:, 6].astype(np.int64) * pieces[:, 7],
+                          minlength=len(chunk_yx))
+    full = covered == ih * iw                            # the boxes are disjoint: areas add up
+    k = np.arange(len(chunk_yx))
+    zero = np.zeros_like(k)
+    below = np.stack([k, zero - 1, ih, zero, zero, zero, cy - ih, zero + cx], 1)[ih < cy]
+    right = np.stack([k, zero - 1, zero, iw, zero, zero, ih, cx - iw], 1)[iw < cx]
+    fill = np.concatenate([below, right])
+    return chunk_yx, pieces, full, np.ascontiguousarray(fill[np.argsort(fill[:, 0], kind='stable')],
+                                                        dtype=np.int32)
+
+
 def _index(key, n, axis):
     """(start, stop, keeps_axis) of one zarr-style basic index along an axis of length ``n``."""
     if isinstance(key, (int, np.integer)) and not isinstance(key, (bool, np.bool_)):
@@ -91,19 +146,68 @@ def _index(key, n, axis):
     raise IndexError('unsupported index %r on axis %d: integers or step-1 slices only' % (key, axis))
 
 
+def _load_model(checkpoint, ps, c):
+    """The model of ``checkpoint`` on the device, checked against chunks of ps x ps x c."""
+    model = AE.autoencoder_from_state_dict(checkpoint, gpu=True, train=False)
+    level = len(model['decoder'].module.synthesis_track)
+    if ps % 2 ** level:
+        raise ValueError('patch size %d is not a multiple of 2^%d' % (ps, level))
+    last = model['decoder'].module.synthesis_track[-1]
+    c_img = last.model[-1].out_channels if hasattr(last, 'model') else 3
+    if c_img != c:
+        raise ValueError('the model reconstructs %d channels, the array has %d' % (c_img, c))
+    return model
+
+
+def create_slide(path, checkpoint, shape, patch_size=512, data_group='0/0', overwrite=False,
+                 **reader_kwargs):
+    """Create an empty Y x X x C ``'cae'`` array and return a ``CompressedSlide`` open for
+    writing (``mode='r+'``; ``reader_kwargs`` go to it).
+
+    The ``.zarray`` is the one ``compress_image`` writes for the same arguments, and no chunk is
+    written, so every chunk reads as the fill value 0 until it is assigned.  Assigning a slide
+    strip by strip, in whole chunks, gives the files ``compress_image`` writes for the whole slide.
+    An existing array is refused unless ``overwrite=True``, which removes its chunks as
+    ``compress_image`` does."""
+    from .compress import _CodecConfig, default_workers
+    arr_path = os.path.join(path, data_group) if data_group else path
+    if os.path.exists(os.path.join(arr_path, '.zarray')) and not overwrite:
+        raise FileExistsError('%s already holds an array (pass overwrite=True to replace it)'
+                              % arr_path)
+    shape = tuple(int(s) for s in shape)
+    ps = int(patch_size)
+    if len(shape) != 3 or min(shape) <= 0 or ps <= 0:
+        raise ValueError('expected a positive Y x X x C shape and patch size, got %r and %d'
+                         % (shape, ps))
+    _load_model(checkpoint, ps, shape[2])         # refuse a mismatched model before writing
+    comp = _CodecConfig('cae', checkpoint=checkpoint if isinstance(checkpoint, str) else '<dict>',
+                        gpu=False)
+    arr = DirArray(arr_path, compressor=comp, mode='w', shape=shape, chunks=(ps, ps, shape[2]),
+                   dtype=np.uint8)
+    arr.remove_chunks(reader_kwargs.get('workers') or default_workers())
+    return CompressedSlide(path, checkpoint, data_group=data_group, mode='r+', **reader_kwargs)
+
+
 class CompressedSlide:
     """Random access to the pixels of a ``'cae'`` array written by ``compress_image``.
 
     ``path``: the store; ``data_group``: the array inside it; ``checkpoint``: the model it was
     compressed with (a path or a state dict); ``batch_tiles``: tiles per synthesis batch (the
-    full batches replay a CUDA graph); ``workers``: native I/O and host coder threads.
+    full batches replay a CUDA graph); ``workers``: native I/O and host coder threads;
+    ``mode``: ``'r'`` (reads only) or ``'r+'`` (reads and writes: ``slide[...] = value``,
+    ``write_region``, ``write_regions``).
 
     The reader owns its model and its device buffers, so it can run beside ``decompress_image``
-    calls on other threads; calls on one reader are serialised.  The decode graphs are captured
-    when the reader is opened."""
+    calls on other threads; calls on one reader are serialised, and a read after a write sees
+    the new chunks.  Several processes may write to one array when their writes cover disjoint
+    whole chunks; two that write a partly covered chunk at once may lose one of the writes (each
+    reads, modifies and replaces the file, with no lock between processes).  The decode graphs
+    (and with ``'r+'`` the encode graphs) are captured when the reader is opened."""
 
-    def __init__(self, path, checkpoint, data_group='0/0', batch_tiles=16, workers=None):
+    def __init__(self, path, checkpoint, data_group='0/0', batch_tiles=16, workers=None, mode='r'):
         from .compress import default_workers
+        if mode not in ('r', 'r+'):
+            raise ValueError("mode must be 'r' or 'r+', got %r" % (mode,))
         if not torch.cuda.is_available():
             raise RuntimeError('CompressedSlide needs a CUDA device (no CPU fallback)')
         self._arr = DirArray(os.path.join(path, data_group) if data_group else path, mode='r')
@@ -118,21 +222,14 @@ class CompressedSlide:
             raise ValueError('expected a Y x X x C uint8 array in square chunks, got shape %r, '
                              'chunks %r, dtype %s' % (self.shape, self.chunks, self.dtype))
         self.ps = int(self.chunks[0])
-        model = AE.autoencoder_from_state_dict(checkpoint, gpu=True, train=False)
-        level = len(model['decoder'].module.synthesis_track)
-        if self.ps % 2 ** level:
-            raise ValueError('patch size %d is not a multiple of 2^%d' % (self.ps, level))
-        last = model['decoder'].module.synthesis_track[-1]
-        c_img = last.model[-1].out_channels if hasattr(last, 'model') else 3
-        if c_img != self.shape[2]:
-            raise ValueError('the model reconstructs %d channels, the array has %d'
-                             % (c_img, self.shape[2]))
+        self.mode = mode
+        model = _load_model(checkpoint, self.ps, self.shape[2])
         self.model = model
         self.fact_ent = model['fact_ent'].module
         self.workers = workers or default_workers()
-        self.tc = _slide.TileCodec(model, self.ps, c_img, int(batch_tiles),
+        self.tc = _slide.TileCodec(model, self.ps, self.shape[2], int(batch_tiles),
                                    graphs=not os.environ.get('CAE_SLIDE_NO_GRAPHS'))
-        self.tc.warm(encode=False, decode=True)
+        self.tc.warm(encode=mode == 'r+', decode=True)
         self._tables = self.fact_ent._host_tables()
         self._pool = None
         self._pieces_dev = None
@@ -153,18 +250,104 @@ class CompressedSlide:
         return self._read(np.array([[y, x]], dtype=np.int64), int(h), int(w), out,
                           (int(h), int(w), self.shape[2]))
 
-    def __getitem__(self, key):
-        """zarr-style basic indexing on Y and X (integers, step-1 slices): a host ndarray."""
+    def _key(self, key):
+        """(y0, y1, x0, x1, keep_y, keep_x) of a zarr-style basic index on Y and X."""
         key = key if isinstance(key, tuple) else (key,)
         if len(key) > 3 or (len(key) == 3 and key[2] != slice(None)):
             raise IndexError('only Y and X can be indexed (the channel axis is read whole)')
         key = tuple(key) + (slice(None),) * (2 - min(len(key), 2))
         y0, y1, keep_y = _index(key[0], self.shape[0], 0)
         x0, x1, keep_x = _index(key[1], self.shape[1], 1)
+        return y0, y1, x0, x1, keep_y, keep_x
+
+    def __getitem__(self, key):
+        """zarr-style basic indexing on Y and X (integers, step-1 slices): a host ndarray."""
+        y0, y1, x0, x1, keep_y, keep_x = self._key(key)
         out = np.empty((y1 - y0, x1 - x0, self.shape[2]), dtype=np.uint8)
         if out.size:
             self.read_region(y0, x0, y1 - y0, x1 - x0, out=out)
         return out[(slice(None) if keep_y else 0, slice(None) if keep_x else 0)]
+
+    # ---- public writes (mode='r+') ----
+    def __setitem__(self, key, value):
+        """zarr-style assignment on Y and X (the index as for ``__getitem__``).  ``value``: a
+        Python int in [0, 255], a uint8 ndarray that broadcasts to the selection, or a contiguous
+        uint8 CUDA tensor of the selection's shape.  Other dtypes are refused rather than cast.
+
+        Like zarr, every chunk the selection touches is read, modified and re-encoded; a chunk
+        the selection covers whole is encoded without reading it, and the re-encoding of a
+        partly covered chunk is lossy (generation loss).  Unlike zarr, the padding of an edge
+        chunk beyond the array edge is always stored as zeros, as ``compress_image`` stores it,
+        so that writing a whole slide gives ``compress_image``'s files."""
+        self._writable()
+        y0, y1, x0, x1, keep_y, keep_x = self._key(key)
+        h, w, c = y1 - y0, x1 - x0, self.shape[2]
+        sel = tuple(n for n, keep in ((h, keep_y), (w, keep_x)) if keep) + (c,)
+        if isinstance(value, (bool, np.bool_)):
+            raise TypeError('bool values are not uint8')
+        if isinstance(value, (int, np.integer)):
+            if not 0 <= int(value) <= 255:
+                raise ValueError('%d does not fit in uint8' % int(value))
+            if h and w:
+                vals = torch.full((1, h, w, c), int(value), dtype=torch.uint8, device=self.tc.dev)
+                self._write(np.array([[y0, x0]], dtype=np.int64), h, w, vals)
+            return
+        if isinstance(value, np.ndarray):
+            if value.dtype != np.uint8:
+                raise ValueError('values must be uint8, got %s (zarr would cast; this does not)'
+                                 % value.dtype)
+            try:
+                value = np.broadcast_to(value, sel)
+            except ValueError:
+                raise ValueError('a value of shape %r does not broadcast to the selection %r'
+                                 % (value.shape, sel)) from None
+            if h and w:
+                self._write(np.array([[y0, x0]], dtype=np.int64), h, w, value.reshape(1, h, w, c))
+            return
+        if isinstance(value, torch.Tensor):
+            if h and w:
+                self._write(np.array([[y0, x0]], dtype=np.int64), h, w,
+                            self._device_values(value, sel).view(1, h, w, c))
+            return
+        raise TypeError('values must be an int, a uint8 ndarray or a uint8 CUDA tensor, got %s'
+                        % type(value).__name__)
+
+    def write_regions(self, boxes, h, w, values):
+        """Write the ``h`` x ``w`` windows with top-left corners ``boxes`` ((y, x) pairs):
+        ``values`` is an N x h x w x c uint8 CUDA tensor or host ndarray (page-locked ones are
+        uploaded asynchronously).  Overlapping boxes are refused before any file is touched.
+        Chunks are re-encoded as for ``__setitem__``."""
+        self._writable()
+        yx = np.asarray(boxes, dtype=np.int64).reshape(-1, 2)
+        shape = (len(yx), int(h), int(w), self.shape[2])
+        if isinstance(values, torch.Tensor):
+            values = self._device_values(values, shape)
+        elif isinstance(values, np.ndarray):
+            if values.dtype != np.uint8 or values.shape != shape:
+                raise ValueError('values must be a uint8 ndarray of shape %r, got %s %r'
+                                 % (shape, values.dtype, values.shape))
+        else:
+            raise TypeError('values must be a uint8 CUDA tensor or host ndarray')
+        self._write(yx, int(h), int(w), values)
+
+    def write_region(self, y, x, value):
+        """Write one h x w x c window at (y, x); ``value`` as one window of ``write_regions``."""
+        self._writable()
+        if not isinstance(value, (torch.Tensor, np.ndarray)) or value.ndim != 3:
+            raise ValueError('value must be an h x w x c uint8 CUDA tensor or host ndarray')
+        self.write_regions([(y, x)], value.shape[0], value.shape[1], value[None])
+
+    def _writable(self):
+        if self.mode != 'r+':
+            raise ValueError("this slide was opened for reading; open it with mode='r+' to write")
+
+    def _device_values(self, t, shape):
+        if (tuple(t.shape) != tuple(shape) or t.dtype != torch.uint8 or t.device != self.tc.dev
+                or not t.is_contiguous()):
+            raise ValueError('values must be a contiguous uint8 tensor of shape %r on %s, got %s '
+                             '%r on %s' % (tuple(shape), self.tc.dev, t.dtype, tuple(t.shape),
+                                           t.device))
+        return t
 
     def close(self):
         if self._pool is not None:
@@ -208,30 +391,86 @@ class CompressedSlide:
                 torch.from_numpy(host_out).copy_(dst)
             return host_out
 
-    def _crop(self, tiles, n_tiles, pieces, dst, n_boxes, h, w):
-        """One ``cae_tiles_crop_u8`` launch on the current stream (the piece table goes up on
-        the same stream, so one device table serves every launch)."""
+    def _table(self, pieces):
+        """The piece table as a contiguous int32 host array, and a device buffer large enough for
+        it (the table goes up on the launch's stream, so one device buffer serves every launch)."""
         if self._pieces_dev is None or self._pieces_dev.numel() < 8 * len(pieces):
             self._pieces_dev = torch.empty(8 * max(1024, len(pieces)), dtype=torch.int32,
                                            device=self.tc.dev)
-        pieces = np.ascontiguousarray(pieces, dtype=np.int32)
+        return np.ascontiguousarray(pieces, dtype=np.int32)
+
+    def _crop(self, tiles, n_tiles, pieces, dst, n_boxes, h, w):
+        """One ``cae_tiles_crop_u8`` launch on the current stream."""
+        pieces = self._table(pieces)
         C.check(C.lib().cae_tiles_crop_u8(
             tiles.data_ptr() if tiles is not None else None, n_tiles, self.ps, self.tc.c_img,
             pieces.ctypes.data, len(pieces), self._pieces_dev.data_ptr(), dst.data_ptr(),
             n_boxes, h, w, _slide._stream_ptr(torch.cuda.current_stream(self.tc.dev))))
 
-    def _decode_and_crop(self, chunk_yx, pieces, dst, n_boxes, h, w):
-        """Decode the chunks ``chunk_yx`` group by group (``_slide.group_sizes``: the symbols of
-        at most one group are on the device) and crop ``pieces`` out of every synthesis batch
-        into ``dst``, on the current stream.  Returns once the device is done."""
-        tc, fe, ps = self.tc, self.fact_ent, self.ps
-        B, dev = tc.batch, tc.dev
-        main = torch.cuda.current_stream(dev)
+    def _paste(self, tiles, n_tiles, pieces, values, h, w):
+        """One ``cae_tiles_paste_u8`` launch on the current stream."""
+        pieces = self._table(pieces)
+        C.check(C.lib().cae_tiles_paste_u8(
+            tiles.data_ptr(), n_tiles, self.ps, self.tc.c_img, pieces.ctypes.data, len(pieces),
+            self._pieces_dev.data_ptr(), values.data_ptr(), values.shape[0], h, w,
+            _slide._stream_ptr(torch.cuda.current_stream(self.tc.dev))))
+
+    def _present(self, chunk_yx):
+        """Chunk file paths of ``chunk_yx`` and which of them exist."""
         paths = [self._arr.chunk_file((int(i), int(j), 0)) for i, j in chunk_yx]
         sizes = np.empty(len(paths), dtype=np.int64)
         C.check(C.lib().cae_files_stat(_paths_blob(paths), len(paths), sizes.ctypes.data,
                                        self.workers))
-        present = sizes >= 0                   # a missing chunk file reads as the fill value 0
+        return paths, sizes >= 0
+
+    def _decode_streams(self, paths, st):
+        """Read the chunk files ``paths`` (one coder group) and entropy-decode their streams:
+        the device coder from ``GPU_CODER_MIN_STREAMS`` streams up, host coder threads below.
+        Returns the int32 symbols n x cb x lh x lw on the device (ready in the current stream's
+        order) and the device coder's status tensor (None for the host coder), which the caller
+        checks once it has synchronised.  Raises before any decode if a header is not the
+        (patch, patch) the codec writes."""
+        tc, fe, dev, gn = self.tc, self.fact_ent, self.tc.dev, len(paths)
+        if self._uploaded is not None:
+            self._uploaded.synchronize()      # the page-locked buffer's last upload has left it
+        hdr, payload, off = native_read(paths, 16, self.workers,
+                                        alloc=lambda n: tc.pinned('region_streams', n).numpy())
+        if bytes(hdr[0]) != struct.pack('>QQ', self.ps, self.ps) or (hdr != hdr[0]).any():
+            raise C.CaeError('chunk headers differ from the (patch, patch) the codec wrote')
+        status = None
+        if gn >= fe.GPU_CODER_MIN_STREAMS:
+            if (off % 4).any():
+                raise C.CaeError('chunk streams are not whole words')
+            words = torch.empty(int(off[-1]) // 4, dtype=torch.int32, device=dev)
+            words.view(torch.uint8).copy_(torch.from_numpy(payload), non_blocking=True)
+            sym, status = fe.decode_streams_device(words, off // 4, tc.lh * tc.lw,
+                                                   defer_status=True)
+            st['device_decoded'] += gn
+        else:
+            # few streams: one host thread per stream beats the device coder's fixed cost
+            cdf, sz, offs = self._tables
+            sym = np.stack(list(self._threads().map(
+                lambda k: decode_symbols(payload[off[k]:off[k + 1]], tc.cb, tc.lh * tc.lw,
+                                         cdf, sz, offs), range(gn))))
+            sym = torch.from_numpy(sym).pin_memory().to(dev, non_blocking=True)
+        self._uploaded = torch.cuda.Event()
+        self._uploaded.record(torch.cuda.current_stream(dev))
+        st['decoded'] += gn
+        return sym.reshape(gn, tc.cb, tc.lh, tc.lw), status
+
+    def _threads(self):
+        if self._pool is None:
+            self._pool = ThreadPoolExecutor(max_workers=self.workers)
+        return self._pool
+
+    def _decode_and_crop(self, chunk_yx, pieces, dst, n_boxes, h, w):
+        """Decode the chunks ``chunk_yx`` group by group (``_slide.group_sizes``: the symbols of
+        at most one group are on the device) and crop ``pieces`` out of every synthesis batch
+        into ``dst``, on the current stream.  Returns once the device is done."""
+        tc, fe = self.tc, self.fact_ent
+        B, dev = tc.batch, tc.dev
+        main = torch.cuda.current_stream(dev)
+        paths, present = self._present(chunk_yx)   # a missing chunk file reads as the fill value 0
         # position of every chunk among the decoded ones (-1: missing), per piece
         piece_tile = np.where(present, np.cumsum(present) - 1, -1)[pieces[:, 0]]
         if not present.all():
@@ -241,39 +480,14 @@ class CompressedSlide:
         todo = [paths[k] for k in np.nonzero(present)[0]]
         self.stats = st = dict(chunks=len(paths), decoded=0, device_decoded=0,
                                missing=len(paths) - len(todo))
-        expect_hdr = struct.pack('>QQ', ps, ps)
         statuses = []
         slot = lo = 0
         groups = _slide.group_sizes(len(todo), _slide.default_schedule(len(todo), B, decode=True),
                                     B) if todo else []
         for gn in groups:
-            if self._uploaded is not None:
-                self._uploaded.synchronize()  # the page-locked buffer's last upload has left it
-            hdr, payload, off = native_read(todo[lo:lo + gn], 16, self.workers,
-                                            alloc=lambda n: tc.pinned('region_streams', n).numpy())
-            if bytes(hdr[0]) != expect_hdr or (hdr != hdr[0]).any():
-                raise C.CaeError('chunk headers differ from the (patch, patch) the codec wrote')
-            if gn >= fe.GPU_CODER_MIN_STREAMS:
-                if (off % 4).any():
-                    raise C.CaeError('chunk streams are not whole words')
-                words = torch.empty(int(off[-1]) // 4, dtype=torch.int32, device=dev)
-                words.view(torch.uint8).copy_(torch.from_numpy(payload), non_blocking=True)
-                sym, status = fe.decode_streams_device(words, off // 4, tc.lh * tc.lw,
-                                                       defer_status=True)
+            sym, status = self._decode_streams(todo[lo:lo + gn], st)
+            if status is not None:
                 statuses.append(status)
-                st['device_decoded'] += gn
-            else:
-                # few streams: one host thread per stream beats the device coder's fixed cost
-                if self._pool is None:
-                    self._pool = ThreadPoolExecutor(max_workers=self.workers)
-                cdf, sz, offs = self._tables
-                sym = np.stack(list(self._pool.map(
-                    lambda k: decode_symbols(payload[off[k]:off[k + 1]], tc.cb, tc.lh * tc.lw,
-                                             cdf, sz, offs), range(gn))))
-                sym = torch.from_numpy(sym).pin_memory().to(dev, non_blocking=True)
-            self._uploaded = torch.cuda.Event()
-            self._uploaded.record(main)
-            sym = sym.reshape(gn, tc.cb, tc.lh, tc.lw)
             for p0 in range(0, gn, B):
                 n = min(B, gn - p0)
                 if n == B and tc.graphs:
@@ -287,8 +501,93 @@ class CompressedSlide:
                 part = pieces[sel]
                 part[:, 0] = piece_tile[sel] - t0
                 self._crop(u8, n, part, dst, n_boxes, h, w)
-            st['decoded'] += gn
             lo += gn
         main.synchronize()
         for status in statuses:
             fe.check_decode_status(status)
+
+    def _write(self, yx, h, w, values):
+        """Write the boxes ``yx`` (``values``: N x h x w x c, on the device or the host) chunk by
+        chunk: group by group (``_slide.group_sizes``), the group's partly covered chunks that
+        have a file are read and decoded, every synthesis-sized batch is assembled in a slot of
+        the codec (decoded tiles, zeros for missing partly covered chunks, then one
+        ``cae_tiles_paste_u8`` launch for the new pixels and the zero padding), encoded, and
+        the group's streams are entropy-coded and written as chunk files (.partial, renamed).
+        Nothing is written before the boxes and values are checked, and a group's files are
+        only written once its old chunks have decoded cleanly."""
+        chunk_yx, pieces, full, fill = write_plan(self.shape, self.chunks, yx, h, w)
+        tc, fe = self.tc, self.fact_ent
+        B, dev = tc.batch, tc.dev
+        with self._lock, torch.cuda.device(dev):
+            main = torch.cuda.current_stream(dev)
+            if isinstance(values, torch.Tensor):
+                vals = values
+            elif _slide.is_pinned_array(values):
+                vals = torch.from_numpy(values).to(dev, non_blocking=True)
+            else:
+                vals = torch.from_numpy(np.ascontiguousarray(values)).to(dev)
+            paths, present = self._present(chunk_yx)
+            # work order: partly covered chunks with a file (decoded), partly covered missing
+            # ones (zeroed), fully covered ones (pasted over whatever the slot held); in every
+            # batch the decoded tiles are then a prefix, moved in with one device copy
+            kind = np.where(full, 2, np.where(present, 0, 1))
+            order = np.argsort(kind, kind='stable')
+            kind = kind[order]
+            pos = np.empty_like(order)
+            pos[order] = np.arange(len(order))
+            table = np.concatenate([pieces, fill])
+            table_pos = pos[table[:, 0]]
+            srt = np.argsort(table_pos, kind='stable')
+            table, table_pos = table[srt], table_pos[srt]
+            K = len(chunk_yx)
+            self.stats = st = dict(chunks=K, full=int(full.sum()), partial=int(K - full.sum()),
+                                   decoded=0, device_decoded=0, missing=int(K - present.sum()),
+                                   device_coded=0)
+            hdr1 = np.frombuffer(struct.pack('>QQ', self.ps, self.ps), dtype=np.uint8)
+            slot = lo = 0
+            for gn in _slide.group_sizes(K, _slide.default_schedule(K, B), B):
+                gd = int((kind[lo:lo + gn] == 0).sum())
+                gz = int((kind[lo:lo + gn] == 1).sum())
+                old, status = (self._decode_streams([paths[k] for k in order[lo:lo + gd]], st)
+                               if gd else (None, None))
+                sym_out = torch.empty((gn, tc.cb, tc.lh * tc.lw), dtype=torch.int32, device=dev)
+                for p0 in range(0, gn, B):
+                    n = min(B, gn - p0)
+                    x = tc.x[slot]
+                    nd = min(max(gd - p0, 0), n)
+                    if nd == B and tc.graphs:
+                        tc.sym_in[slot].copy_(old[p0:p0 + nd], non_blocking=True)
+                        x.copy_(tc.decode(slot, nd), non_blocking=True)
+                    elif nd:
+                        x[:nd].copy_(tc.decode_eager(old[p0:p0 + nd]), non_blocking=True)
+                    nz = min(max(gd + gz - p0, 0), n) - nd
+                    if nz:
+                        x[nd:nd + nz].zero_()
+                    a, b = np.searchsorted(table_pos, [lo + p0, lo + p0 + n])
+                    part = table[a:b].copy()
+                    part[:, 0] = table_pos[a:b] - (lo + p0)
+                    self._paste(x, n, part, vals, h, w)
+                    sym_out[p0:p0 + n].copy_(tc.encode(slot, n).reshape(n, tc.cb, -1),
+                                             non_blocking=True)
+                    slot = (slot + 1) % tc.slots
+                if gn >= fe.GPU_CODER_MIN_STREAMS:
+                    packed, off = fe.encode_symbols_device(sym_out)
+                    host = tc.pinned('region_write_streams', packed.numel())
+                    host.copy_(packed, non_blocking=True)
+                    main.synchronize()
+                    payload = host.numpy()
+                    st['device_coded'] += gn
+                else:
+                    sym_h = sym_out.cpu().numpy()
+                    cdf, sz, offs = self._tables
+                    streams = list(self._threads().map(
+                        lambda k: encode_symbols(sym_h[k], cdf, sz, offs), range(gn)))
+                    off = np.zeros(gn + 1, dtype=np.int64)
+                    np.cumsum([len(s) for s in streams], out=off[1:])
+                    payload = np.frombuffer(b''.join(streams), dtype=np.uint8)
+                if status is not None:
+                    fe.check_decode_status(status)
+                native_write([paths[k] for k in order[lo:lo + gn]], np.broadcast_to(hdr1, (gn, 16)),
+                             payload, off, self.workers)
+                lo += gn
+            main.synchronize()

@@ -409,6 +409,15 @@ int cae_tiles_crop_u8(const uint8_t *tiles, int n_tiles, int ps, int c,
                       const int32_t *pieces /*HOST, m x 8*/, int m, int32_t *pieces_dev /*m x 8*/,
                       uint8_t *out, int n_boxes, int box_h, int box_w, void *stream);
 
+/* Region writes: the inverse.  The same piece table, read the other way: rows [dy, dy+h) x columns
+ * [dx, dx+w) of box b of `boxes` (n_boxes x box_h x box_w x c) go to (sy, sx) of tile k of `tiles`;
+ * b = -1 writes zeros instead (the padding of an edge chunk; dy, dx are then ignored).  The pieces
+ * of one call must not overlap in `tiles`.  Checked on the host like cae_tiles_crop_u8; bytes of
+ * `tiles` outside the pieces are left as they are.                                             */
+int cae_tiles_paste_u8(uint8_t *tiles, int n_tiles, int ps, int c,
+                       const int32_t *pieces /*HOST, m x 8*/, int m, int32_t *pieces_dev /*m x 8*/,
+                       const uint8_t *boxes, int n_boxes, int box_h, int box_w, void *stream);
+
 /* ---- evaluation sums on the device (SURVEY.md 8f-4) ------------------------------------------ */
 /* sse[i] += sum over the per_image uint8 values of image i of (a - b)^2: the numerator of
  * compute_rmse / compute_psnr (src/test_cae.py:57-63, computed there on the host after a full
