@@ -81,7 +81,10 @@ typedef struct {
   const float *bias;       /* c_out floats or NULL                                       */
   int32_t pre_act, post_act;
   int32_t pad_mode;        /* direct kernel only (CAE_PAD_*); igemm reads the halo       */
-  int32_t ck;              /* igemm: channels per K chunk (16/32/48/64), 0 = auto        */
+  int32_t ck;              /* igemm: channels per K chunk (16/32/48/64/128 dividing c_in
+                              padded to 16), 0 = auto; a ck whose activation stage and two
+                              weight stages exceed shared memory is refused (e.g. 128 on a
+                              stride-1 layer of 128 -> 192 channels, 64 on a stride-2 one)  */
   int32_t mt;              /* igemm: 16x8 M-tiles per CTA tile (1/2), 0 = auto           */
   int32_t grid;            /* igemm: CTAs, 0 = one per SM                                */
   void *aux_out;           /* optional second output (fp32 NCHW) or NULL                 */
@@ -121,7 +124,11 @@ int cae_pack_weights(int kind, int c_in, int c_out, int ck, const float *w,
  * inside Analyzer.forward R:359-361 and Synthesizer.forward R:442-455.        */
 int cae_conv_igemm(const cae_conv_desc *d, void *stream);
 /* CUDA-core direct path for the thin image-side layers (c_in < 16: the 3->3
- * stem, R:63-70 with channels_org) and tiny nets; any format combination.     */
+ * stem, R:63-70 with channels_org) and tiny nets; any format combination.
+ * PLANAR / SPLIT outputs: the dense stride-1 form with c_in, c_out <= 4 (the tiled
+ * stem) writes plane 0 only (its padded channels as +0) and leaves further planes
+ * as allocated, so they must hold zeros (alloc_act clears them); every other form
+ * writes all `planes`, padded channels as +0.                                    */
 int cae_conv_direct(const cae_conv_desc *d, void *stream);
 
 /* Fused head of an analysis track: the first DownsamplingUnit of the reference
