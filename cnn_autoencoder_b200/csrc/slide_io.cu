@@ -8,6 +8,8 @@
 // the caller's stream, so uploads, kernels and downloads of neighbouring batches overlap.
 #include "cae_common.cuh"
 
+#include <vector>
+
 // dst[k] (device, ps x ps x c, tile-major) = tile (tile_yx[2k], tile_yx[2k+1]) of the host image;
 // the part of an edge tile beyond the image is zero (zarr's chunk padding, fill_value 0).
 extern "C" int cae_tiles_upload_u8(const uint8_t *src, int64_t H, int64_t W, int c, int ps,
@@ -285,6 +287,217 @@ extern "C" int cae_tiles_paste_u8(uint8_t *tiles, int n_tiles, int ps, int c,
                            cudaMemcpyHostToDevice, st));
   tiles_paste_u8_kernel<<<grid, kCropThreads, 0, st>>>(
       tiles, ps, c, reinterpret_cast<const int4 *>(pieces_dev), boxes, box_h, box_w, rows);
+  cae_count_launch();
+  CAE_CUDA(cudaGetLastError());
+  return 0;
+}
+
+// ---------------------------------------------------------------------------------------------
+// Reduced-resolution region reads (region.SlideLevel).  A piece is the crop's record in level-f
+// pixels followed by the in-array extent of tile k in level-0 pixels: {k, b, sy, sx, dy, dx, h, w,
+// vh, vw, 0, 0}.  Level pixel (i, j) of tile k, channel ch, is the mean, rounded half up, of
+// level-0 rows [i f, min((i + 1) f, vh)) x columns [j f, min((j + 1) f, vw)) of the tile: the
+// decoded padding of an edge tile never enters a mean.  k = -1 writes zeros.
+//
+// Bound by the source bytes it reads (a batch of decoded tiles, just written by the synthesis and
+// L2-resident); the output is 1/f^2 of them.  Block (p, q, r) covers nb output rows x wb output
+// columns of piece p, sized to read ~32 KB.  Its threads own VEC-byte units of the source rows
+// (16 where the tiles allow) and split the f source rows of each output row among `split` thread
+// groups: each thread sums its rows of its unit in registers and adds the sums into the block's
+// column sums in shared memory.  Then groups of g lanes each add part of one output element's f
+// columns (stride c in shared memory: no bank conflicts for odd c) and finish with shuffles.
+namespace {
+constexpr int kReduceThreads = 256;
+constexpr int kReduceSource = 32768;   // source bytes per block
+constexpr int kReduceSpan = 4096;      // source bytes per row of a block, unless one pixel is wider
+constexpr int kReduceSmem = 40960;     // column sums per block, bytes
+
+template <int VEC>
+__device__ __forceinline__ void add_unit(const uint8_t *p, uint32_t (&acc)[VEC]) {
+  if constexpr (VEC == 16) {
+    const uint4 v = __ldg(reinterpret_cast<const uint4 *>(p));
+    const uint32_t wd[4] = {v.x, v.y, v.z, v.w};
+#pragma unroll
+    for (int i = 0; i < 16; ++i) acc[i] += (wd[i >> 2] >> (8 * (i & 3))) & 255u;
+  } else if constexpr (VEC == 4) {
+    const uint32_t v = __ldg(reinterpret_cast<const uint32_t *>(p));
+#pragma unroll
+    for (int i = 0; i < 4; ++i) acc[i] += (v >> (8 * i)) & 255u;
+  } else {
+    acc[0] += __ldg(p);
+  }
+}
+
+// n / d as a multiply-high by m = magic(d) = ceil(2^32 / d): exact while n * d < 2^32
+__device__ __forceinline__ uint32_t magic(uint32_t d) { return d == 1 ? 0u : 0xFFFFFFFFu / d + 1; }
+__device__ __forceinline__ uint32_t div_by(uint32_t n, uint32_t d, uint32_t m) {
+  return d == 1 ? n : __umulhi(n, m);
+}
+
+template <int VEC>
+__global__ void __launch_bounds__(kReduceThreads, 4) tiles_crop_reduce_u8_kernel(
+    const uint8_t *__restrict__ tiles, int ps, int c, int lf, const int4 *__restrict__ pieces,
+    uint8_t *__restrict__ out, int box_h, int box_w, int nb, int wb, int g) {
+  extern __shared__ uint32_t colsum[];
+  const int4 p0 = pieces[3 * blockIdx.x], p1 = pieces[3 * blockIdx.x + 1],
+             p2 = pieces[3 * blockIdx.x + 2];
+  const int k = p0.x, b = p0.y, sy = p0.z, sx = p0.w, dy = p1.x, dx = p1.y, h = p1.z, w = p1.w;
+  const int vh = p2.x, vw = p2.y;
+  const int o0 = blockIdx.y * nb, j0 = blockIdx.z * wb;
+  if (o0 >= h || j0 >= w) return;
+  const int f = 1 << lf, rows = min(nb, h - o0), cols = min(wb, w - j0);
+  const int row_out = cols * c, n_out = rows * row_out;
+  uint8_t *dst = out + (((size_t)b * box_h + dy + o0) * box_w + dx + j0) * c;
+  const size_t dst_pitch = (size_t)box_w * c;
+  if (k < 0) {
+    for (int e = threadIdx.x; e < n_out; e += kReduceThreads) {
+      const int o = e / row_out;
+      dst[o * dst_pitch + e - o * row_out] = 0;
+    }
+    return;
+  }
+  // bytes [a0, end) of every source row: the block's columns, from a VEC-aligned start
+  const int a0 = (((sx + j0) << lf) * c) & ~(VEC - 1);
+  const int end = min((sx + j0 + cols) << lf, vw) * c;
+  const int units = (end - a0 + VEC - 1) / VEC, stride = units * VEC;
+  // vertical: item (rg, o, u) sums rows rg, rg + split, ... < f of output row o, unit u.  Threads
+  // share an (o, u) only when there are too few of them to fill the block (large f); then the
+  // sums meet through shared-memory atomics, else each (o, u) has one writer.
+  const int pairs = rows * units;
+  int split = 1;
+  while (split < f && 2 * split * pairs <= kReduceThreads) split *= 2;
+  if (split > 1) {
+    for (int i = threadIdx.x; i < rows * stride; i += kReduceThreads) colsum[i] = 0;
+    __syncthreads();
+  }
+  const int row0 = (sy + o0) << lf;
+  const int src_rows = min(rows << lf, vh - row0);           // the band's rows inside the array
+  const size_t pitch = (size_t)ps * c;
+  const uint8_t *src = tiles + ((size_t)k * ps + row0) * pitch + a0;
+  const uint32_t m_units = magic(units), m_rows = magic(rows);
+  for (int i = threadIdx.x; i < pairs * split; i += kReduceThreads) {
+    const int q = (int)div_by(i, units, m_units), u = i - q * units;
+    const int rg = (int)div_by(q, rows, m_rows), o = q - rg * rows;
+    const int t_end = min(f, src_rows - (o << lf));
+    uint32_t acc[VEC] = {};
+#pragma unroll 2
+    for (int t = rg; t < t_end; t += split)
+      add_unit<VEC>(src + (size_t)((o << lf) + t) * pitch + u * VEC, acc);
+    uint32_t *cs = colsum + o * stride + u * VEC;
+    if (split == 1) {
+#pragma unroll
+      for (int v = 0; v < VEC; ++v) cs[v] = acc[v];
+    } else if (rg < t_end) {
+#pragma unroll
+      for (int v = 0; v < VEC; ++v) atomicAdd(cs + v, acc[v]);
+    }
+  }
+  __syncthreads();
+  // horizontal: g lanes per output element, each adding every g-th of its columns
+  const int lane = threadIdx.x & (g - 1), per_pass = kReduceThreads / g;
+  const uint32_t m_row = magic(row_out), m_c = magic(c);
+  for (int e0 = 0; e0 < n_out; e0 += per_pass) {
+    const int e = e0 + threadIdx.x / g;
+    uint32_t s = 0;
+    int o = 0, r = 0, nc = f, nr = f;
+    if (e < n_out) {
+      o = (int)div_by(e, row_out, m_row);
+      r = e - o * row_out;
+      const int jj = (int)div_by(r, c, m_c), ch = r - jj * c;
+      const int col0 = (sx + j0 + jj) << lf;
+      nc = min(f, vw - col0);
+      nr = min(f, vh - row0 - (o << lf));
+      const uint32_t *cs = colsum + o * stride + col0 * c + ch - a0;
+      for (int t = lane; t < nc; t += g) s += cs[t * c];
+    }
+    for (int off = g >> 1; off > 0; off >>= 1) s += __shfl_xor_sync(0xffffffffu, s, off);
+    if (e < n_out && lane == 0) {
+      const uint32_t n = (uint32_t)nc * (uint32_t)nr;      // f^2 except in edge blocks
+      dst[o * dst_pitch + r] = (uint8_t)(n == (1u << 2 * lf) ? (s + n / 2) >> 2 * lf : (s + n / 2) / n);
+    }
+  }
+}
+}  // namespace
+
+extern "C" int cae_tiles_crop_reduce_u8(const uint8_t *tiles, int n_tiles, int ps, int c, int f,
+                                        const int32_t *pieces, int m, int32_t *pieces_dev,
+                                        uint8_t *out, int n_boxes, int box_h, int box_w,
+                                        void *stream) {
+  const char *fn = "cae_tiles_crop_reduce_u8";
+  CAE_CHECK(n_tiles >= 0 && ps > 0 && c > 0 && m >= 0 && n_boxes > 0 && box_h > 0 && box_w > 0, 2,
+            "%s: bad argument", fn);
+  CAE_CHECK(f >= 1 && f <= 512 && (f & (f - 1)) == 0 && ps % f == 0, 2,
+            "%s: the factor %d is not a power of two in [1, 512] that divides the tile size %d", fn,
+            f, ps);
+  CAE_CHECK((int64_t)ps * ps * c <= INT32_MAX && (int64_t)box_w * c <= INT32_MAX, 2,
+            "%s: tile or box row too large", fn);
+  CAE_CHECK(((int64_t)f * c + 32) * 4 <= kReduceSmem, 2, "%s: %d x %d bytes per pixel is too wide",
+            fn, f, c);
+  if (m == 0) return 0;
+  CAE_CHECK(pieces && pieces_dev && out && (tiles || n_tiles == 0), 2, "%s: null pointer", fn);
+  CAE_CHECK((uintptr_t)pieces_dev % 16 == 0, 2, "%s: pieces_dev is not 16-byte aligned", fn);
+  const int lps = ps / f;
+  int max_h = 0, max_w = 0;
+  for (int i = 0; i < m; ++i) {
+    const int32_t *p = pieces + 12 * (size_t)i;
+    const int k = p[0], b = p[1], sy = p[2], sx = p[3], dy = p[4], dx = p[5], h = p[6], w = p[7];
+    const int vh = p[8], vw = p[9];
+    CAE_CHECK(k >= -1 && k < n_tiles, 2, "%s: piece %d names tile %d of %d", fn, i, k, n_tiles);
+    CAE_CHECK(b >= 0 && b < n_boxes, 2, "%s: piece %d names box %d of %d", fn, i, b, n_boxes);
+    CAE_CHECK(h > 0 && w > 0 && sy >= 0 && sx >= 0 && sy <= lps - h && sx <= lps - w, 2,
+              "%s: piece %d (rows %d+%d, columns %d+%d) lies outside its %d^2 level tile", fn, i,
+              sy, h, sx, w, lps);
+    CAE_CHECK(vh > 0 && vw > 0 && vh <= ps && vw <= ps, 2,
+              "%s: piece %d: in-array extent %d x %d of a %d^2 tile", fn, i, vh, vw, ps);
+    CAE_CHECK((int64_t)(sy + h - 1) * f < vh && (int64_t)(sx + w - 1) * f < vw, 2,
+              "%s: piece %d (rows %d+%d, columns %d+%d) starts past the in-array part %d x %d",
+              fn, i, sy, h, sx, w, vh, vw);
+    CAE_CHECK(dy >= 0 && dx >= 0 && dy <= box_h - h && dx <= box_w - w, 2,
+              "%s: piece %d (rows %d+%d, columns %d+%d) lies outside its %d x %d box", fn, i, dy,
+              h, dx, w, box_h, box_w);
+    max_h = h > max_h ? h : max_h;
+    max_w = w > max_w ? w : max_w;
+  }
+  if (f == 1) {   // the level image is the slide itself: the crop kernel copies in wide units
+    std::vector<int32_t> p8(8 * (size_t)m);
+    for (int i = 0; i < m; ++i)
+      for (int j = 0; j < 8; ++j) p8[8 * (size_t)i + j] = pieces[12 * (size_t)i + j];
+    return cae_tiles_crop_u8(tiles, n_tiles, ps, c, p8.data(), m, pieces_dev, out, n_boxes, box_h,
+                             box_w, stream);
+  }
+  const int vec = tiles == nullptr ? 16
+                  : ((uintptr_t)tiles | (uintptr_t)ps * c) % 16 == 0 ? 16
+                  : ((uintptr_t)tiles | (uintptr_t)ps * c) % 4 == 0  ? 4 : 1;
+  // a block: ~kReduceSource source bytes, rows of at most kReduceSpan bytes (or one pixel)
+  const int fc = f * c;
+  int span = kReduceSource / f < kReduceSpan ? kReduceSource / f : kReduceSpan;
+  int wb = (span > fc ? span : fc) / fc;
+  wb = wb < max_w ? wb : max_w;
+  const int row_smem = (wb * fc + 2 * vec) * 4;
+  int nb = kReduceSource / (f * wb * fc);
+  nb = nb < kReduceSmem / row_smem ? nb : kReduceSmem / row_smem;
+  nb = nb < max_h ? nb : max_h;
+  nb = nb < 1 ? 1 : nb;
+  const int gy = (max_h + nb - 1) / nb, gz = (max_w + wb - 1) / wb;
+  CAE_CHECK(gy <= 65535 && gz <= 65535, 2, "%s: pieces of %d x %d are too large", fn, max_h, max_w);
+  int lf = 0;
+  while ((1 << lf) < f) ++lf;
+  const int g = f / 4 < 1 ? 1 : f / 4 > 32 ? 32 : f / 4;
+  cudaStream_t st = (cudaStream_t)stream;
+  CAE_CUDA(cudaMemcpyAsync(pieces_dev, pieces, sizeof(int32_t) * 12 * (size_t)m,
+                           cudaMemcpyHostToDevice, st));
+  const dim3 grid((unsigned)m, (unsigned)gy, (unsigned)gz);
+  const size_t smem = (size_t)nb * row_smem;
+  const int4 *pd = reinterpret_cast<const int4 *>(pieces_dev);
+  if (vec == 16)
+    tiles_crop_reduce_u8_kernel<16><<<grid, kReduceThreads, smem, st>>>(tiles, ps, c, lf, pd, out,
+                                                                        box_h, box_w, nb, wb, g);
+  else if (vec == 4)
+    tiles_crop_reduce_u8_kernel<4><<<grid, kReduceThreads, smem, st>>>(tiles, ps, c, lf, pd, out,
+                                                                       box_h, box_w, nb, wb, g);
+  else
+    tiles_crop_reduce_u8_kernel<1><<<grid, kReduceThreads, smem, st>>>(tiles, ps, c, lf, pd, out,
+                                                                       box_h, box_w, nb, wb, g);
   cae_count_launch();
   CAE_CUDA(cudaGetLastError());
   return 0;

@@ -12,6 +12,10 @@ the synthesis transform over ``batch_tiles`` tiles at a time with the kernels of
 engine, and after every batch one launch of ``cae_tiles_crop_u8`` cuts the boxes' pieces out of
 the decoded tiles on the device.  The pixels are the ones ``decompress_image`` writes.
 
+``CompressedSlide.downsampled(f)`` (``SlideLevel``) reads the slide at 1/f of its resolution, as
+a viewer or a 20x / 10x patch sampler wants it: the same decode, and after every batch one launch
+of ``cae_tiles_crop_reduce_u8`` box-filters the pieces (``reduce_plan``) into the level image.
+
 Opened with ``mode='r+'`` (or made empty by ``create_slide``) it also writes, as zarr's
 assignment does: a read-modify-write per touched chunk.  ``write_plan`` adds to ``plan`` which
 chunks are covered whole (encoded without reading them) and the zero pieces of edge padding; the
@@ -146,6 +150,60 @@ def _index(key, n, axis):
     raise IndexError('unsupported index %r on axis %d: integers or step-1 slices only' % (key, axis))
 
 
+def _basic_key(key, shape):
+    """(y0, y1, x0, x1, keep_y, keep_x) of a zarr-style basic index on Y and X of ``shape``."""
+    key = key if isinstance(key, tuple) else (key,)
+    if len(key) > 3 or (len(key) == 3 and key[2] != slice(None)):
+        raise IndexError('only Y and X can be indexed (the channel axis is read whole)')
+    key = tuple(key) + (slice(None),) * (2 - min(len(key), 2))
+    y0, y1, keep_y = _index(key[0], shape[0], 0)
+    x0, x1, keep_x = _index(key[1], shape[1], 1)
+    return y0, y1, x0, x1, keep_y, keep_x
+
+
+def _getitem(arr, key):
+    """``arr[key]`` as a host ndarray through ``arr.read_region`` (basic indexing on Y and X)."""
+    y0, y1, x0, x1, keep_y, keep_x = _basic_key(key, arr.shape)
+    out = np.empty((y1 - y0, x1 - x0, arr.shape[2]), dtype=np.uint8)
+    if out.size:
+        arr.read_region(y0, x0, y1 - y0, x1 - x0, out=out)
+    return out[(slice(None) if keep_y else 0, slice(None) if keep_x else 0)]
+
+
+def level_shape(shape, f):
+    """Shape of the level-``f`` image of a Y x X x c array: ceil(Y/f) x ceil(X/f) x c."""
+    return (-(-int(shape[0]) // f), -(-int(shape[1]) // f)) + tuple(int(s) for s in shape[2:])
+
+
+def check_factor(f, ps):
+    """``f`` as an int; ``ValueError`` unless it is a power of two with 1 <= f <= ps, ps % f == 0."""
+    if isinstance(f, (bool, np.bool_)) or not isinstance(f, (int, np.integer)):
+        raise ValueError('the downsample factor must be an int, got %r' % (f,))
+    f = int(f)
+    if f < 1 or f & (f - 1) or ps % f:
+        raise ValueError('the downsample factor must be a power of two that divides the chunk '
+                         'size %d, got %d' % (ps, f))
+    return f
+
+
+def reduce_plan(shape, ps, f, boxes, box_h, box_w):
+    """``plan`` for boxes of the level-``f`` image of a Y x X x c array in ps^2 chunks.
+
+    Every level pixel lies in one chunk (ps % f == 0), so the level image is stored in chunks of
+    ps/f that correspond one to one with the level-0 chunks: ``chunk_yx`` names the same files.
+    Returns ``(chunk_yx, pieces)`` with int32 P x 12 pieces ``{k, b, sy, sx, dy, dx, h, w, vh, vw,
+    0, 0}``: ``plan``'s record in level pixels and the in-array extent of chunk k in level-0
+    pixels, the record ``cae_tiles_crop_reduce_u8`` reads."""
+    f = check_factor(f, ps)
+    chunk_yx, p8 = plan(level_shape(shape, f), (ps // f, ps // f), boxes, box_h, box_w)
+    iy, ix = chunk_yx[p8[:, 0], 0], chunk_yx[p8[:, 0], 1]
+    pieces = np.zeros((len(p8), 12), dtype=np.int32)
+    pieces[:, :8] = p8
+    pieces[:, 8] = np.minimum(ps, int(shape[0]) - iy * ps)
+    pieces[:, 9] = np.minimum(ps, int(shape[1]) - ix * ps)
+    return chunk_yx, pieces
+
+
 def _load_model(checkpoint, ps, c):
     """The model of ``checkpoint`` on the device, checked against chunks of ps x ps x c."""
     model = AE.autoencoder_from_state_dict(checkpoint, gpu=True, train=False)
@@ -250,23 +308,15 @@ class CompressedSlide:
         return self._read(np.array([[y, x]], dtype=np.int64), int(h), int(w), out,
                           (int(h), int(w), self.shape[2]))
 
-    def _key(self, key):
-        """(y0, y1, x0, x1, keep_y, keep_x) of a zarr-style basic index on Y and X."""
-        key = key if isinstance(key, tuple) else (key,)
-        if len(key) > 3 or (len(key) == 3 and key[2] != slice(None)):
-            raise IndexError('only Y and X can be indexed (the channel axis is read whole)')
-        key = tuple(key) + (slice(None),) * (2 - min(len(key), 2))
-        y0, y1, keep_y = _index(key[0], self.shape[0], 0)
-        x0, x1, keep_x = _index(key[1], self.shape[1], 1)
-        return y0, y1, x0, x1, keep_y, keep_x
-
     def __getitem__(self, key):
         """zarr-style basic indexing on Y and X (integers, step-1 slices): a host ndarray."""
-        y0, y1, x0, x1, keep_y, keep_x = self._key(key)
-        out = np.empty((y1 - y0, x1 - x0, self.shape[2]), dtype=np.uint8)
-        if out.size:
-            self.read_region(y0, x0, y1 - y0, x1 - x0, out=out)
-        return out[(slice(None) if keep_y else 0, slice(None) if keep_x else 0)]
+        return _getitem(self, key)
+
+    def downsampled(self, f):
+        """A read-only view of the slide at 1/``f`` of its resolution (``SlideLevel``): ``f`` is a
+        power of two that divides the chunk size.  It shares this reader's model, buffers and
+        lock, and reads see this reader's writes."""
+        return SlideLevel(self, f)
 
     # ---- public writes (mode='r+') ----
     def __setitem__(self, key, value):
@@ -280,7 +330,7 @@ class CompressedSlide:
         chunk beyond the array edge is always stored as zeros, as ``compress_image`` stores it,
         so that writing a whole slide gives ``compress_image``'s files."""
         self._writable()
-        y0, y1, x0, x1, keep_y, keep_x = self._key(key)
+        y0, y1, x0, x1, keep_y, keep_x = _basic_key(key, self.shape)
         h, w, c = y1 - y0, x1 - x0, self.shape[2]
         sel = tuple(n for n, keep in ((h, keep_y), (w, keep_x)) if keep) + (c,)
         if isinstance(value, (bool, np.bool_)):
@@ -361,8 +411,13 @@ class CompressedSlide:
         self.close()
 
     # ---- the work ----
-    def _read(self, yx, h, w, out, shape):
-        chunk_yx, pieces = plan(self.shape, self.chunks, yx, h, w)
+    def _read(self, yx, h, w, out, shape, f=1):
+        """The boxes ``yx`` of the level-``f`` image (f = 1: the slide) into ``out``."""
+        n_boxes = len(yx)
+        if f == 1:
+            chunk_yx, pieces = plan(self.shape, self.chunks, yx, h, w)
+        else:
+            chunk_yx, pieces = reduce_plan(self.shape, self.ps, f, yx, h, w)
         dev = self.tc.dev
         host_out = None
         if out is None:
@@ -380,8 +435,14 @@ class CompressedSlide:
             dst = torch.empty(shape, dtype=torch.uint8, device=dev)
         else:
             raise TypeError('out must be a CUDA tensor or a host ndarray')
+        if f == 1:
+            def step(tiles, n_tiles, part):
+                self._crop(tiles, n_tiles, part, dst, n_boxes, h, w)
+        else:
+            def step(tiles, n_tiles, part):
+                self._crop_reduce(tiles, n_tiles, f, part, dst, n_boxes, h, w)
         with self._lock, torch.cuda.device(dev):
-            self._decode_and_crop(chunk_yx, pieces, dst, len(yx), h, w)
+            self._decode_and_crop(chunk_yx, pieces, step)
             if host_out is None:
                 return dst
             if _slide.is_pinned_array(host_out):
@@ -394,8 +455,8 @@ class CompressedSlide:
     def _table(self, pieces):
         """The piece table as a contiguous int32 host array, and a device buffer large enough for
         it (the table goes up on the launch's stream, so one device buffer serves every launch)."""
-        if self._pieces_dev is None or self._pieces_dev.numel() < 8 * len(pieces):
-            self._pieces_dev = torch.empty(8 * max(1024, len(pieces)), dtype=torch.int32,
+        if self._pieces_dev is None or self._pieces_dev.numel() < pieces.size:
+            self._pieces_dev = torch.empty(max(8 * 1024, pieces.size), dtype=torch.int32,
                                            device=self.tc.dev)
         return np.ascontiguousarray(pieces, dtype=np.int32)
 
@@ -404,6 +465,14 @@ class CompressedSlide:
         pieces = self._table(pieces)
         C.check(C.lib().cae_tiles_crop_u8(
             tiles.data_ptr() if tiles is not None else None, n_tiles, self.ps, self.tc.c_img,
+            pieces.ctypes.data, len(pieces), self._pieces_dev.data_ptr(), dst.data_ptr(),
+            n_boxes, h, w, _slide._stream_ptr(torch.cuda.current_stream(self.tc.dev))))
+
+    def _crop_reduce(self, tiles, n_tiles, f, pieces, dst, n_boxes, h, w):
+        """One ``cae_tiles_crop_reduce_u8`` launch on the current stream (``pieces``: P x 12)."""
+        pieces = self._table(pieces)
+        C.check(C.lib().cae_tiles_crop_reduce_u8(
+            tiles.data_ptr() if tiles is not None else None, n_tiles, self.ps, self.tc.c_img, f,
             pieces.ctypes.data, len(pieces), self._pieces_dev.data_ptr(), dst.data_ptr(),
             n_boxes, h, w, _slide._stream_ptr(torch.cuda.current_stream(self.tc.dev))))
 
@@ -463,10 +532,12 @@ class CompressedSlide:
             self._pool = ThreadPoolExecutor(max_workers=self.workers)
         return self._pool
 
-    def _decode_and_crop(self, chunk_yx, pieces, dst, n_boxes, h, w):
+    def _decode_and_crop(self, chunk_yx, pieces, step):
         """Decode the chunks ``chunk_yx`` group by group (``_slide.group_sizes``: the symbols of
-        at most one group are on the device) and crop ``pieces`` out of every synthesis batch
-        into ``dst``, on the current stream.  Returns once the device is done."""
+        at most one group are on the device) and hand every synthesis batch with its ``pieces``
+        to ``step(tiles, n_tiles, part)`` on the current stream (``part[:, 0]`` indexes the
+        batch; the pieces of missing chunks come first, with ``tiles`` None and k = -1).
+        Returns once the device is done."""
         tc, fe = self.tc, self.fact_ent
         B, dev = tc.batch, tc.dev
         main = torch.cuda.current_stream(dev)
@@ -476,7 +547,7 @@ class CompressedSlide:
         if not present.all():
             fill = pieces[piece_tile < 0].copy()
             fill[:, 0] = -1
-            self._crop(None, 0, fill, dst, n_boxes, h, w)
+            step(None, 0, fill)
         todo = [paths[k] for k in np.nonzero(present)[0]]
         self.stats = st = dict(chunks=len(paths), decoded=0, device_decoded=0,
                                missing=len(paths) - len(todo))
@@ -500,7 +571,7 @@ class CompressedSlide:
                 sel = (piece_tile >= t0) & (piece_tile < t0 + n)
                 part = pieces[sel]
                 part[:, 0] = piece_tile[sel] - t0
-                self._crop(u8, n, part, dst, n_boxes, h, w)
+                step(u8, n, part)
             lo += gn
         main.synchronize()
         for status in statuses:
@@ -591,3 +662,44 @@ class CompressedSlide:
                              payload, off, self.workers)
                 lo += gn
             main.synchronize()
+
+
+class SlideLevel:
+    """The slide at 1/``f`` of its resolution (``CompressedSlide.downsampled(f)``), read-only.
+
+    The level-``f`` image of a Y x X x c slide is ceil(Y/f) x ceil(X/f) x c.  Its pixel (i, j),
+    channel ch, is the mean, rounded half up, of the slide's pixels in rows [i f, min((i+1) f, Y))
+    x columns [j f, min((j+1) f, X)): what PIL's ``Image.reduce(f)`` computes on whole blocks,
+    while edge blocks average only the pixels inside the array.  A missing chunk reads as 0.
+
+    Reads decode the chunks they touch exactly as the slide's own reads do (same files, coder
+    groups, synthesis batches, lock and ``stats``); after every synthesis batch one
+    ``cae_tiles_crop_reduce_u8`` launch writes the batch's pieces of the level image, so no
+    buffer of the level-0 window exists.  ``f`` = 1 reads the slide through its own path."""
+
+    def __init__(self, slide, f):
+        self.downsample = check_factor(f, slide.ps)
+        self._slide = slide
+        self.shape = level_shape(slide.shape, self.downsample)
+        self.chunks = (slide.ps // self.downsample,) * 2 + (slide.shape[2],)
+        self.dtype = slide.dtype
+
+    def read_regions(self, boxes, h, w, out=None):
+        """The ``h`` x ``w`` windows at ``boxes`` of the level image; as the slide's
+        ``read_regions``, in level pixels."""
+        yx = np.asarray(boxes, dtype=np.int64).reshape(-1, 2)
+        return self._slide._read(yx, int(h), int(w), out, (len(yx), int(h), int(w), self.shape[2]),
+                                 self.downsample)
+
+    def read_region(self, y, x, h, w, out=None):
+        """One ``h`` x ``w`` x c window at (y, x) of the level image; ``out`` as for
+        ``read_regions``."""
+        return self._slide._read(np.array([[y, x]], dtype=np.int64), int(h), int(w), out,
+                                 (int(h), int(w), self.shape[2]), self.downsample)
+
+    def __getitem__(self, key):
+        """zarr-style basic indexing on Y and X of the level image: a host ndarray."""
+        return _getitem(self, key)
+
+    def __setitem__(self, key, value):
+        raise TypeError('a downsampled view is read-only: write to the slide it was taken from')

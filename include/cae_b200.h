@@ -425,6 +425,21 @@ int cae_tiles_paste_u8(uint8_t *tiles, int n_tiles, int ps, int c,
                        const int32_t *pieces /*HOST, m x 8*/, int m, int32_t *pieces_dev /*m x 8*/,
                        const uint8_t *boxes, int n_boxes, int box_h, int box_w, void *stream);
 
+/* Reduced-resolution region reads: windows of the level-f image cut out of one batch of decoded
+ * tiles.  f is a power of two in [1, 512] that divides ps; level pixel (i, j) of tile k, channel
+ * ch, is the mean, rounded half up ((s + n/2) / n over the n pixels), of level-0 rows
+ * [i f, min((i+1) f, vh)) x columns [j f, min((j+1) f, vw)) of the tile.  Piece i =
+ * pieces[12i .. 12i+11] = {k, b, sy, sx, dy, dx, h, w, vh, vw, 0, 0}: the crop's record in level
+ * pixels (tile k's level grid is (ps/f)^2; `out` is n_boxes x box_h x box_w x c level pixels) and
+ * the in-array extent 0 < vh, vw <= ps of tile k in level-0 pixels (ps, except for edge chunks;
+ * the padding beyond it never enters a mean; (sy+h-1) f < vh and (sx+w-1) f < vw).  k = -1 writes
+ * zeros.  Checked on the host like cae_tiles_crop_u8; `pieces_dev`: DEVICE, m x 12 int32,
+ * 16-byte aligned.                                                                             */
+int cae_tiles_crop_reduce_u8(const uint8_t *tiles, int n_tiles, int ps, int c, int f,
+                             const int32_t *pieces /*HOST, m x 12*/, int m,
+                             int32_t *pieces_dev /*m x 12*/, uint8_t *out, int n_boxes, int box_h,
+                             int box_w, void *stream);
+
 /* ---- evaluation sums on the device (SURVEY.md 8f-4) ------------------------------------------ */
 /* sse[i] += sum over the per_image uint8 values of image i of (a - b)^2: the numerator of
  * compute_rmse / compute_psnr (src/test_cae.py:57-63, computed there on the host after a full
