@@ -33,7 +33,7 @@ SYMBOLS = ['cae_abi_version', 'cae_last_error', 'cae_device_info', 'cae_launch_c
            'cae_tiles_download_u8_banded', 'cae_sse_u8', 'cae_ssim_u8', 'cae_delta_e_u8', 'cae_u8_to_planes_f32',
            'cae_avgpool2_planes_f32', 'cae_ssim_gauss_planes_f32', 'cae_tiles_gather_u8', 'cae_files_write', 'cae_files_stat', 'cae_files_read',
            'cae_files_remove', 'cae_tiles_crop_u8', 'cae_tiles_paste_u8',
-           'cae_tiles_crop_reduce_u8']
+           'cae_tiles_crop_reduce_u8', 'cae_tiles_pyramid_u8']
 
 
 class Tensor(ctypes.Structure):
@@ -199,6 +199,7 @@ def lib():
     L.cae_tiles_crop_u8.argtypes = [vp, ci, ci, ci, vp, ci, vp, vp, ci, ci, ci, vp]
     L.cae_tiles_paste_u8.argtypes = [vp, ci, ci, ci, vp, ci, vp, vp, ci, ci, ci, vp]
     L.cae_tiles_crop_reduce_u8.argtypes = [vp, ci, ci, ci, ci, vp, ci, vp, vp, ci, ci, ci, vp]
+    L.cae_tiles_pyramid_u8.argtypes = [vp, ci, ci, ci, ci, vp, vp, ci, ci, vp, vp]
     for name in SYMBOLS:
         if name not in ('cae_abi_version', 'cae_last_error', 'cae_launch_count',
                         'cae_packed_weight_bytes', 'cae_rans_enc_table_bytes',

@@ -504,6 +504,170 @@ extern "C" int cae_tiles_crop_reduce_u8(const uint8_t *tiles, int n_tiles, int p
 }
 
 // ---------------------------------------------------------------------------------------------
+// Resolution pyramid (region.CompressedSlide.build_pyramid): levels 1..K of a batch of decoded
+// tiles in one launch, each tile read once.  Record t = {i, j, vh, vw}: tile t is level-0 chunk
+// (i, j) with in-array extent vh x vw; the chunks of one call lie in one level-1 chunk row (equal
+// i >> 1, hence equal i >> k at every level), since `out` holds one chunk row per level.  Its level-k pixels, the same means as
+// cae_tiles_crop_reduce_u8 at f = 2^k, land in tile j >> k of level k's chunk-row buffer at
+// ((i mod 2^k) ps/2^k, (j mod 2^k) ps/2^k); only the ceil(vh/2^k) x ceil(vw/2^k) pixels inside
+// the array are written.
+//
+// Block (q, t) covers a Q x Q square of tile t, Q = max(2^K, S): every level pixel of the square
+// lies in it, so no sum crosses blocks.  The block stages S x S level-0 squares (S = 64 or the
+// largest power of two dividing ps, if smaller) in shared memory one at a time, zeroing the
+// pixels outside the array, and builds the 2 x 2 sums level by level in shared memory (integer
+// sums of level-0 pixels at every level, never means of means), storing each level's means as it
+// goes.  The S x S totals then feed the levels above log2 S the same way.
+namespace {
+constexpr int kPyrThreads = 256;
+constexpr int kPyrMaxLevels = 9;
+constexpr int kPyrSmem = 48 * 1024;
+
+struct PyrLevels {
+  int off[kPyrMaxLevels + 1];   // off[k]: first tile of level k's chunk-row buffer in `out`
+};
+
+// Level-l pixel (py, px) of the tile (level-l pixels, tile-local), channel ch, from its sum s.
+__device__ __forceinline__ void pyr_store(uint8_t *__restrict__ out, const int *off, int ps,
+                                          int c, int l, int i, int j, int vh, int vw, int py,
+                                          int px, int ch, uint32_t s) {
+  const int y0 = py << l, x0 = px << l;
+  if (y0 >= vh || x0 >= vw) return;
+  const uint32_t n = (uint32_t)min(1 << l, vh - y0) * (uint32_t)min(1 << l, vw - x0);
+  const int lps = ps >> l, mask = (1 << l) - 1;
+  const size_t row = (size_t)(i & mask) * lps + py, col = (size_t)(j & mask) * lps + px;
+  uint8_t *t = out + (size_t)(off[l] + (j >> l)) * ps * ps * c;
+  t[(row * ps + col) * c + ch] =
+      (uint8_t)(n == (1u << 2 * l) ? (s + n / 2) >> 2 * l : (s + n / 2) / n);
+}
+
+// dst (n/2 x n/2 x c) = the 2 x 2 sums of src (n x n x c): level l, whose pixel (y, x) is level-l
+// pixel (py0 + y, px0 + x) of the tile.
+template <typename T>
+__device__ __forceinline__ void pyr_level(const T *src, uint32_t *dst, int n, int c,
+                                          uint8_t *__restrict__ out, const int *off, int ps,
+                                          int l, int i, int j, int vh, int vw, int py0, int px0) {
+  const int h = n >> 1, lh = 31 - __clz(h), m = (h * h) * c;
+  for (int e = threadIdx.x; e < m; e += kPyrThreads) {
+    const int q = e / c, ch = e - q * c, y = q >> lh, x = q & (h - 1);
+    const T *s0 = src + ((size_t)(2 * y) * n + 2 * x) * c + ch;
+    const uint32_t s = (uint32_t)s0[0] + (uint32_t)s0[c] + (uint32_t)s0[n * c] +
+                       (uint32_t)s0[n * c + c];
+    dst[e] = s;
+    pyr_store(out, off, ps, c, l, i, j, vh, vw, py0 + y, px0 + x, ch, s);
+  }
+  __syncthreads();
+}
+
+template <int VEC>
+__global__ void __launch_bounds__(kPyrThreads) tiles_pyramid_u8_kernel(
+    const uint8_t *__restrict__ tiles, int ps, int c, int levels, int ls, int lq,
+    const int4 *__restrict__ recs, uint8_t *__restrict__ out, PyrLevels lv) {
+  extern __shared__ __align__(16) uint8_t pyr_smem[];
+  __shared__ int off[kPyrMaxLevels + 1];
+  if (threadIdx.x <= kPyrMaxLevels) off[threadIdx.x] = lv.off[threadIdx.x];
+  const int4 r = recs[blockIdx.y];
+  const int i = r.x, j = r.y, vh = r.z, vw = r.w;
+  const int S = 1 << ls, Q = 1 << lq, per_row = ps >> lq;
+  const int Y0 = (blockIdx.x / per_row) << lq, X0 = (blockIdx.x % per_row) << lq;
+  if (Y0 >= vh || X0 >= vw) return;          // no pixel of the square is inside the array
+  const int row_b = S * c;
+  uint8_t *px = pyr_smem;                                                   // S x S x c bytes
+  uint32_t *a = reinterpret_cast<uint32_t *>(pyr_smem + ((S * row_b + 15) & ~15));
+  uint32_t *b = a + (S / 2) * (S / 2) * c;                                  // (S/4)^2 x c
+  uint32_t *top = b + (S / 4) * (S / 4) * c;                                // (Q/S)^2 x c
+  uint32_t *top2 = top + (Q / S) * (Q / S) * c;                             // (Q/2S)^2 x c
+  const int nsub = Q >> ls, l_in = min(levels, ls);
+  const uint8_t *tile = tiles + (size_t)blockIdx.y * ps * ps * c;
+  const int units = row_b / VEC;
+  for (int s = 0; s < nsub * nsub; ++s) {
+    const int y0 = Y0 + (s / nsub) * S, x0 = X0 + (s % nsub) * S;
+    const int v_rows = vh - y0, v_bytes = (vw - x0) * c;     // inside the array (may be <= 0)
+    for (int u = threadIdx.x; u < S * units; u += kPyrThreads) {
+      const int rr = u / units, b0 = (u - rr * units) * VEC;
+      const uint8_t *g = tile + ((size_t)(y0 + rr) * ps + x0) * c + b0;
+      uint8_t *d = px + rr * row_b + b0;
+      if (VEC == 16 && rr < v_rows && b0 + 16 <= v_bytes) {
+        *reinterpret_cast<uint4 *>(d) = __ldg(reinterpret_cast<const uint4 *>(g));
+      } else {
+#pragma unroll
+        for (int v = 0; v < VEC; ++v) d[v] = rr < v_rows && b0 + v < v_bytes ? __ldg(g + v) : 0;
+      }
+    }
+    __syncthreads();
+    pyr_level<uint8_t>(px, a, S, c, out, off, ps, 1, i, j, vh, vw, y0 >> 1, x0 >> 1);
+    uint32_t *src = a, *dst = b;
+    for (int l = 2; l <= l_in; ++l) {
+      pyr_level<uint32_t>(src, dst, S >> (l - 1), c, out, off, ps, l, i, j, vh, vw, y0 >> l,
+                          x0 >> l);
+      uint32_t *t = src; src = dst; dst = t;
+    }
+    // the square's totals (src is 1 x 1 x c when levels > ls); the next square's staging
+    // barrier orders this read before `a` and `b` are written again
+    if (levels > ls && threadIdx.x < c) top[s * c + threadIdx.x] = src[threadIdx.x];
+  }
+  if (levels > ls) {
+    __syncthreads();
+    uint32_t *src = top, *dst = top2;
+    for (int l = ls + 1; l <= levels; ++l) {
+      pyr_level<uint32_t>(src, dst, nsub >> (l - ls - 1), c, out, off, ps, l, i, j, vh, vw,
+                          Y0 >> l, X0 >> l);
+      uint32_t *t = src; src = dst; dst = t;
+    }
+  }
+}
+}  // namespace
+
+extern "C" int cae_tiles_pyramid_u8(const uint8_t *tiles, int n_tiles, int ps, int c, int levels,
+                                    const int32_t *recs, int32_t *recs_dev, int gy, int gx,
+                                    uint8_t *out, void *stream) {
+  const char *fn = "cae_tiles_pyramid_u8";
+  CAE_CHECK(n_tiles >= 0 && n_tiles <= 65535 && ps > 0 && c > 0 && gy > 0 && gx > 0, 2,
+            "%s: bad argument", fn);
+  CAE_CHECK(levels >= 1 && levels <= kPyrMaxLevels && ps % (1 << levels) == 0, 2,
+            "%s: %d levels: K must be in [1, %d] with 2^K dividing the tile size %d", fn, levels,
+            kPyrMaxLevels, ps);
+  CAE_CHECK((int64_t)ps * ps * c <= INT32_MAX, 2, "%s: tile too large", fn);
+  int ls = 0;                 // S = 2^ls: min(64, the largest power of two dividing ps)
+  while (ls < 6 && ps % (2 << ls) == 0) ++ls;
+  const int lq = levels > ls ? levels : ls;
+  const int64_t S = 1 << ls, nsub = 1 << (lq - ls);
+  const int64_t smem = ((S * S * c + 15) & ~15) +
+                       4 * c * (S * S / 4 + S * S / 16 + nsub * nsub + nsub * nsub / 4);
+  CAE_CHECK(smem <= kPyrSmem, 2, "%s: %d channels need %lld bytes of shared memory", fn, c,
+            (long long)smem);
+  if (n_tiles == 0) return 0;
+  CAE_CHECK(tiles && recs && recs_dev && out, 2, "%s: null pointer", fn);
+  CAE_CHECK((uintptr_t)recs_dev % 16 == 0, 2, "%s: recs_dev is not 16-byte aligned", fn);
+  for (int t = 0; t < n_tiles; ++t) {
+    const int32_t *p = recs + 4 * (size_t)t;
+    CAE_CHECK(p[0] >= 0 && p[0] < gy && p[1] >= 0 && p[1] < gx, 2,
+              "%s: record %d names chunk (%d, %d) of a %d x %d grid", fn, t, p[0], p[1], gy, gx);
+    CAE_CHECK(p[2] > 0 && p[2] <= ps && p[3] > 0 && p[3] <= ps, 2,
+              "%s: record %d: in-array extent %d x %d of a %d^2 tile", fn, t, p[2], p[3], ps);
+    CAE_CHECK(p[0] >> 1 == recs[0] >> 1, 2,
+              "%s: record %d (chunk row %d) and record 0 (chunk row %d) are in different level-1 "
+              "chunk rows", fn, t, p[0], recs[0]);
+  }
+  PyrLevels lv = {};
+  for (int l = 1; l < levels; ++l) lv.off[l + 1] = lv.off[l] + (gx + (1 << l) - 1) / (1 << l);
+  cudaStream_t st = (cudaStream_t)stream;
+  CAE_CUDA(cudaMemcpyAsync(recs_dev, recs, sizeof(int32_t) * 4 * (size_t)n_tiles,
+                           cudaMemcpyHostToDevice, st));
+  const dim3 grid((unsigned)((ps >> lq) * (ps >> lq)), (unsigned)n_tiles);
+  const int4 *rd = reinterpret_cast<const int4 *>(recs_dev);
+  if (((uintptr_t)tiles | (uintptr_t)(S * c)) % 16 == 0)
+    tiles_pyramid_u8_kernel<16><<<grid, kPyrThreads, (size_t)smem, st>>>(tiles, ps, c, levels, ls,
+                                                                         lq, rd, out, lv);
+  else
+    tiles_pyramid_u8_kernel<1><<<grid, kPyrThreads, (size_t)smem, st>>>(tiles, ps, c, levels, ls,
+                                                                        lq, rd, out, lv);
+  cae_count_launch();
+  CAE_CUDA(cudaGetLastError());
+  return 0;
+}
+
+// ---------------------------------------------------------------------------------------------
 // Evaluation sums on the device (SURVEY.md 8f-4; src/test_cae.py:60-63 PSNR, :57-58 RMSE and the
 // distortion term of src/models/criteria/_ratedist.py:57-63 in uint8 units): per image
 //   sse[i] += sum (a - b)^2   over the `per_image` uint8 values of image i.

@@ -25,6 +25,7 @@ group and written as chunk files.  The padding of an edge chunk is always stored
 (``compress_image`` does the same; zarr would keep the decoded padding), so writing a slide in
 whole chunks gives ``compress_image``'s files byte for byte.
 """
+import json
 import os
 import struct
 import threading
@@ -204,6 +205,97 @@ def reduce_plan(shape, ps, f, boxes, box_h, box_w):
     return chunk_yx, pieces
 
 
+def check_levels(levels, ps):
+    """``levels`` (K) as an int; ``ValueError`` unless K >= 1 and 2^K divides the chunk size."""
+    if isinstance(levels, (bool, np.bool_)) or not isinstance(levels, (int, np.integer)):
+        raise ValueError('levels must be an int, got %r' % (levels,))
+    K = int(levels)
+    if K < 1 or K > 30:
+        raise ValueError('levels must be at least 1, got %d' % K)
+    check_factor(2 ** K, ps)
+    return K
+
+
+def default_levels(shape, ps):
+    """The smallest K >= 1 whose level image fits in one ps^2 chunk, capped at the largest K with
+    2^K dividing ps (log2 ps for a power of two)."""
+    cap = 0
+    while ps % 2 ** (cap + 1) == 0:
+        cap += 1
+    K = 1
+    while K < cap and max(level_shape(shape, 2 ** K)[:2]) > ps:
+        K += 1
+    return K
+
+
+def pyramid_rows(gy, levels):
+    """The level chunk rows in the order a pass over the gy level-0 chunk rows completes them:
+    (k, R) once level-0 row 2^k (R + 1) - 1, or the last row, has been reduced."""
+    return [(k, i >> k) for i in range(gy) for k in range(1, levels + 1)
+            if (i + 1) % 2 ** k == 0 or i == gy - 1]
+
+
+def pyramid_place(shape, ps, k, chunk_yx):
+    """Where ``cae_tiles_pyramid_u8`` puts level-0 chunks ``chunk_yx`` (K x 2) of a Y x X array in
+    ps^2 chunks at level k: int64 K x 5 ``{tile, oy, ox, eh, ew}``: tile column ``tile`` of level
+    k's chunk row i >> k, at (oy, ox) in that tile, an in-array extent of eh x ew level pixels."""
+    ij = np.asarray(chunk_yx, dtype=np.int64).reshape(-1, 2)
+    i, j = ij[:, 0], ij[:, 1]
+    f, lps = 2 ** k, ps >> k
+    vh = np.minimum(ps, int(shape[0]) - i * ps)
+    vw = np.minimum(ps, int(shape[1]) - j * ps)
+    return np.stack([j >> k, (i % f) * lps, (j % f) * lps, -(-vh // f), -(-vw // f)], 1)
+
+
+def multiscales(levels, name=''):
+    """The OME-Zarr 0.4 style ``multiscales`` entry of levels 0..K (axes y, x, c)."""
+    return [{'version': '0.4', 'name': name,
+             'axes': [{'name': 'y', 'type': 'space'}, {'name': 'x', 'type': 'space'},
+                      {'name': 'c', 'type': 'channel'}],
+             'datasets': [{'path': str(k), 'coordinateTransformations':
+                           [{'type': 'scale', 'scale': [2 ** k, 2 ** k, 1]}]}
+                          for k in range(levels + 1)],
+             'type': 'mean'}]
+
+
+def _write_json(path, obj):
+    """``obj`` as JSON at ``path``, written aside and renamed: readers never see a partial file."""
+    tmp = path + '.%d.tmp' % os.getpid()
+    with open(tmp, 'w') as f:
+        json.dump(obj, f, indent=1)
+    os.replace(tmp, path)
+
+
+def _read_attrs(group):
+    try:
+        with open(os.path.join(group, '.zattrs')) as f:
+            return json.load(f)
+    except FileNotFoundError:
+        return {}
+
+
+def stored_levels(group):
+    """The level paths (ints) listed by the ``multiscales`` entry of ``<group>/.zattrs``; [0]
+    without one."""
+    ms = _read_attrs(group).get('multiscales')
+    if not ms:
+        return [0]
+    return [int(d['path']) for d in ms[0]['datasets']]
+
+
+def write_multiscales(store, group, levels):
+    """``.zgroup`` at the store root and at ``group`` where absent, and the ``multiscales`` entry
+    of levels 0..K in ``<group>/.zattrs`` (its other keys are kept; levels=0 removes the entry)."""
+    for d in {os.path.normpath(store), os.path.normpath(group)}:
+        if not os.path.exists(os.path.join(d, '.zgroup')):
+            _write_json(os.path.join(d, '.zgroup'), {'zarr_format': 2})
+    attrs = _read_attrs(group)
+    attrs.pop('multiscales', None)
+    if levels:
+        attrs['multiscales'] = multiscales(levels)
+    _write_json(os.path.join(group, '.zattrs'), attrs)
+
+
 def _load_model(checkpoint, ps, c):
     """The model of ``checkpoint`` on the device, checked against chunks of ps x ps x c."""
     model = AE.autoencoder_from_state_dict(checkpoint, gpu=True, train=False)
@@ -269,6 +361,8 @@ class CompressedSlide:
         if not torch.cuda.is_available():
             raise RuntimeError('CompressedSlide needs a CUDA device (no CPU fallback)')
         self._arr = DirArray(os.path.join(path, data_group) if data_group else path, mode='r')
+        self._store = path
+        self._data_group = data_group
         codec_id = (self._arr.compressor_config or {}).get('id')
         if codec_id == 'cae_bn':
             raise ValueError("the array stores latents ('cae_bn'): its chunks are not pixels; "
@@ -294,6 +388,8 @@ class CompressedSlide:
         self._uploaded = None             # the last upload out of the page-locked stream buffer
         self._lock = threading.Lock()
         self.stats = {}
+        group = self._pyramid_group()
+        self.levels = stored_levels(group) if group is not None else [0]
 
     # ---- public reads ----
     def read_regions(self, boxes, h, w, out=None):
@@ -317,6 +413,165 @@ class CompressedSlide:
         power of two that divides the chunk size.  It shares this reader's model, buffers and
         lock, and reads see this reader's writes."""
         return SlideLevel(self, f)
+
+    def level(self, k):
+        """A read-only view of the stored pyramid level ``k`` (``<group>/k``, see
+        ``build_pyramid``; ``StoredLevel``): the level's own chunks, read with this reader's
+        model, buffers, lock and ``stats``.  ``level(0)`` is the slide itself.  Raises
+        ``KeyError`` for a level that is not stored."""
+        if isinstance(k, (bool, np.bool_)) or not isinstance(k, (int, np.integer)):
+            raise TypeError('the level must be an int, got %r' % (k,))
+        if int(k) not in self.levels:
+            raise KeyError('level %d is not stored (stored levels: %s)' % (int(k), self.levels))
+        return self if int(k) == 0 else StoredLevel(self, int(k))
+
+    def _pyramid_group(self):
+        """The directory holding the levels (``<group>`` of a ``<group>/0`` data group), or None
+        when the data group's last component is not ``0``."""
+        parts = [p for p in (self._data_group or '').split('/') if p]
+        if not parts or parts[-1] != '0':
+            return None
+        return os.path.join(self._store, *parts[:-1])
+
+    def build_pyramid(self, levels=None, overwrite=False):
+        """Write the resolution pyramid: level k = 1..K as a ``'cae'`` array ``<group>/k`` beside
+        the slide's ``<group>/0``, and a ``multiscales`` entry listing levels 0..K in
+        ``<group>/.zattrs`` (``.zgroup`` files where absent).  Needs ``mode='r+'``.
+
+        Level k holds ``self.downsampled(2 ** k)[:]`` (block means of the decoded slide, rounded
+        half up; edge blocks average the pixels inside the array) encoded in ps^2 chunks with the
+        slide's codec config: its ``.zarray`` and chunk files are the ones ``compress_image``
+        writes for that image.  Reading a stored level (``level(k)``) decodes a few of its
+        chunks instead of every level-0 chunk under the window, but its pixels went through one
+        more lossy encode; ``downsampled(f)`` stays the exact mean of level 0.
+
+        ``levels``: K, default the smallest K whose level fits in one chunk (capped at log2 ps).
+        The slide is decoded once, group by group; after every synthesis batch one
+        ``cae_tiles_pyramid_u8`` launch per level-0 chunk row in the batch reduces each decoded
+        tile into every level, and each
+        level chunk row is encoded, entropy-coded and written as soon as its last level-0 row has
+        been reduced, so only one chunk row per level is ever held.  ``self.stats['decoded']``
+        counts the level-0 chunk files read.
+
+        The metadata follows OME-Zarr 0.4 ``multiscales`` (datasets with ``scale`` transforms
+        [2^k, 2^k, 1], ``"type": "mean"``) with one difference: the axes are y, x, c, channel
+        last as ``compress_image`` stores the slide, where OME-NGFF 0.4 puts the channel axis
+        before the spatial ones.  The entry is written last, once every level file is; with
+        ``overwrite=True`` the old entry is removed first, then the old levels' chunks, so a
+        reader never finds a listed level with incomplete files.
+
+        Later writes to the slide (``slide[...] = v``) do not update the levels: rebuild with
+        ``overwrite=True`` after them.  Refused, before any file is touched: a reader opened with
+        ``'r'``, K < 1 or 2^K not dividing ps, a data group whose last component is not ``0``,
+        and existing level arrays unless ``overwrite=True``."""
+        from .compress import _CodecConfig
+        self._writable()
+        ps, c = self.ps, self.shape[2]
+        K = default_levels(self.shape, ps) if levels is None else check_levels(levels, ps)
+        group = self._pyramid_group()
+        if group is None:
+            raise ValueError("the levels go beside a '<group>/0' array; this slide's data group "
+                             "is %r" % (self._data_group,))
+        level_paths = [os.path.join(group, str(k)) for k in range(1, K + 1)]
+        existing = [q for q in level_paths if os.path.exists(os.path.join(q, '.zarray'))]
+        if existing and not overwrite:
+            raise FileExistsError('%s already holds a level array (pass overwrite=True to rebuild)'
+                                  % existing[0])
+        tc, B, dev = self.tc, self.tc.batch, self.tc.dev
+        Y, X = self.shape[:2]
+        gy, gx = self._arr.grid[:2]
+        with self._lock, torch.cuda.device(dev):
+            if overwrite:
+                if 'multiscales' in _read_attrs(group):
+                    write_multiscales(self._store, group, 0)
+                    self.levels = [0]
+                for q in existing:
+                    DirArray(q, mode='r').remove_chunks(self.workers)
+            cfg = dict(self._arr.compressor_config)
+            comp = _CodecConfig(cfg.pop('id'), **cfg)
+            arrs = {k: DirArray(q, compressor=comp, mode='w', shape=level_shape(self.shape, 2 ** k),
+                                chunks=(ps, ps, c), dtype=np.uint8)
+                    for k, q in zip(range(1, K + 1), level_paths)}
+            for a in arrs.values():
+                a.remove_chunks(self.workers)
+            # one chunk row per level, back to back: the layout cae_tiles_pyramid_u8 writes
+            widths = [-(-gx // 2 ** k) for k in range(1, K + 1)]
+            first = np.concatenate([[0], np.cumsum(widths)])
+            rows = torch.zeros((int(first[-1]), ps, ps, c), dtype=torch.uint8, device=dev)
+            order = pyramid_rows(gy, K)
+            paths = [arrs[k].chunk_file((R, col, 0)) for k, R in order
+                     for col in range(widths[k - 1])]
+            groups = iter(_slide.group_sizes(len(paths), _slide.default_schedule(len(paths), B),
+                                             B))
+            st = dict(level_chunks=len(paths), device_coded=0)
+            enc = dict(slot=0, fill=0, lo=0, gn=next(groups), g0=0, sym=None)
+
+            def encode_slot():
+                e = enc
+                n = e['fill']
+                e['sym'][e['g0']:e['g0'] + n].copy_(tc.encode(e['slot'], n).reshape(n, tc.cb, -1),
+                                                    non_blocking=True)
+                e['g0'] += n
+                e['slot'], e['fill'] = (e['slot'] + 1) % tc.slots, 0
+                if e['g0'] == e['gn']:
+                    self._code_and_write(e['sym'], paths[e['lo']:e['lo'] + e['gn']], st)
+                    e['lo'] += e['gn']
+                    e['gn'], e['g0'], e['sym'] = next(groups, 0), 0, None
+
+            def flush(k):
+                """Hand level k's finished chunk row to the encoder and clear it."""
+                row = rows[first[k - 1]:first[k]]
+                a = 0
+                while a < len(row):
+                    e = enc
+                    if e['sym'] is None:
+                        e['sym'] = torch.empty((e['gn'], tc.cb, tc.lh * tc.lw), dtype=torch.int32,
+                                               device=dev)
+                    m = min(len(row) - a, B - e['fill'], e['gn'] - e['g0'] - e['fill'])
+                    tc.x[e['slot']][e['fill']:e['fill'] + m].copy_(row[a:a + m], non_blocking=True)
+                    e['fill'] += m
+                    a += m
+                    if e['fill'] == B or e['g0'] + e['fill'] == e['gn']:
+                        encode_slot()
+                row.zero_()
+
+            done = [0]                   # level-0 chunk rows reduced so far
+
+            def complete(upto):
+                for i in range(done[0], upto):
+                    for k in range(1, K + 1):
+                        if (i + 1) % 2 ** k == 0 or i == gy - 1:
+                            flush(k)
+                done[0] = max(done[0], upto)
+
+            tile_bytes = ps * ps * c
+
+            def step(tiles, n_tiles, part):
+                if tiles is None:        # missing chunks: their level pixels are the zeros rows holds
+                    return
+                # one launch per level-0 chunk row of the batch: the rows before it are complete
+                # (chunks come in row-major order) and leave the buffers before its tiles land
+                cuts = np.flatnonzero(np.diff(part[:, 1])) + 1
+                for a, b in zip(np.concatenate([[0], cuts]), np.concatenate([cuts, [n_tiles]])):
+                    complete(int(part[a, 1]))
+                    recs = self._table(part[a:b, 1:5])
+                    C.check(C.lib().cae_tiles_pyramid_u8(
+                        tiles.data_ptr() + int(a) * tile_bytes, int(b - a), ps, c, K,
+                        recs.ctypes.data, self._pieces_dev.data_ptr(), gy, gx, rows.data_ptr(),
+                        _slide._stream_ptr(torch.cuda.current_stream(dev))))
+                complete(int(part[-1, 1]) + (int(part[-1, 2]) == gx - 1))
+
+            ii, jj = np.meshgrid(np.arange(gy), np.arange(gx), indexing='ij')
+            chunk_yx = np.stack([ii.ravel(), jj.ravel()], 1)
+            pieces = np.stack([np.arange(len(chunk_yx)), chunk_yx[:, 0], chunk_yx[:, 1],
+                               np.minimum(ps, Y - chunk_yx[:, 0] * ps),
+                               np.minimum(ps, X - chunk_yx[:, 1] * ps)], 1).astype(np.int32)
+            self._decode_and_crop(chunk_yx, pieces, step)
+            complete(gy)
+            torch.cuda.current_stream(dev).synchronize()
+            self.stats.update(st)
+            write_multiscales(self._store, group, K)
+            self.levels = list(range(K + 1))
 
     # ---- public writes (mode='r+') ----
     def __setitem__(self, key, value):
@@ -411,11 +666,13 @@ class CompressedSlide:
         self.close()
 
     # ---- the work ----
-    def _read(self, yx, h, w, out, shape, f=1):
-        """The boxes ``yx`` of the level-``f`` image (f = 1: the slide) into ``out``."""
+    def _read(self, yx, h, w, out, shape, f=1, arr=None):
+        """The boxes ``yx`` of the level-``f`` image (f = 1: the slide, or the stored array
+        ``arr``) into ``out``."""
         n_boxes = len(yx)
+        arr = self._arr if arr is None else arr
         if f == 1:
-            chunk_yx, pieces = plan(self.shape, self.chunks, yx, h, w)
+            chunk_yx, pieces = plan(arr.shape, arr.chunks, yx, h, w)
         else:
             chunk_yx, pieces = reduce_plan(self.shape, self.ps, f, yx, h, w)
         dev = self.tc.dev
@@ -442,7 +699,7 @@ class CompressedSlide:
             def step(tiles, n_tiles, part):
                 self._crop_reduce(tiles, n_tiles, f, part, dst, n_boxes, h, w)
         with self._lock, torch.cuda.device(dev):
-            self._decode_and_crop(chunk_yx, pieces, step)
+            self._decode_and_crop(chunk_yx, pieces, step, arr)
             if host_out is None:
                 return dst
             if _slide.is_pinned_array(host_out):
@@ -484,9 +741,10 @@ class CompressedSlide:
             self._pieces_dev.data_ptr(), values.data_ptr(), values.shape[0], h, w,
             _slide._stream_ptr(torch.cuda.current_stream(self.tc.dev))))
 
-    def _present(self, chunk_yx):
-        """Chunk file paths of ``chunk_yx`` and which of them exist."""
-        paths = [self._arr.chunk_file((int(i), int(j), 0)) for i, j in chunk_yx]
+    def _present(self, chunk_yx, arr=None):
+        """Chunk file paths of ``chunk_yx`` (of ``arr``, default the slide) and which of them
+        exist."""
+        paths = [(self._arr if arr is None else arr).chunk_file((int(i), int(j), 0)) for i, j in chunk_yx]
         sizes = np.empty(len(paths), dtype=np.int64)
         C.check(C.lib().cae_files_stat(_paths_blob(paths), len(paths), sizes.ctypes.data,
                                        self.workers))
@@ -532,8 +790,8 @@ class CompressedSlide:
             self._pool = ThreadPoolExecutor(max_workers=self.workers)
         return self._pool
 
-    def _decode_and_crop(self, chunk_yx, pieces, step):
-        """Decode the chunks ``chunk_yx`` group by group (``_slide.group_sizes``: the symbols of
+    def _decode_and_crop(self, chunk_yx, pieces, step, arr=None):
+        """Decode the chunks ``chunk_yx`` (of ``arr``, default the slide) group by group (``_slide.group_sizes``: the symbols of
         at most one group are on the device) and hand every synthesis batch with its ``pieces``
         to ``step(tiles, n_tiles, part)`` on the current stream (``part[:, 0]`` indexes the
         batch; the pieces of missing chunks come first, with ``tiles`` None and k = -1).
@@ -541,7 +799,7 @@ class CompressedSlide:
         tc, fe = self.tc, self.fact_ent
         B, dev = tc.batch, tc.dev
         main = torch.cuda.current_stream(dev)
-        paths, present = self._present(chunk_yx)   # a missing chunk file reads as the fill value 0
+        paths, present = self._present(chunk_yx, arr)   # a missing chunk reads as the fill value 0
         # position of every chunk among the decoded ones (-1: missing), per piece
         piece_tile = np.where(present, np.cumsum(present) - 1, -1)[pieces[:, 0]]
         if not present.all():
@@ -614,7 +872,6 @@ class CompressedSlide:
             self.stats = st = dict(chunks=K, full=int(full.sum()), partial=int(K - full.sum()),
                                    decoded=0, device_decoded=0, missing=int(K - present.sum()),
                                    device_coded=0)
-            hdr1 = np.frombuffer(struct.pack('>QQ', self.ps, self.ps), dtype=np.uint8)
             slot = lo = 0
             for gn in _slide.group_sizes(K, _slide.default_schedule(K, B), B):
                 gd = int((kind[lo:lo + gn] == 0).sum())
@@ -641,28 +898,37 @@ class CompressedSlide:
                     sym_out[p0:p0 + n].copy_(tc.encode(slot, n).reshape(n, tc.cb, -1),
                                              non_blocking=True)
                     slot = (slot + 1) % tc.slots
-                if gn >= fe.GPU_CODER_MIN_STREAMS:
-                    packed, off = fe.encode_symbols_device(sym_out)
-                    host = tc.pinned('region_write_streams', packed.numel())
-                    host.copy_(packed, non_blocking=True)
-                    main.synchronize()
-                    payload = host.numpy()
-                    st['device_coded'] += gn
-                else:
-                    sym_h = sym_out.cpu().numpy()
-                    cdf, sz, offs = self._tables
-                    streams = list(self._threads().map(
-                        lambda k: encode_symbols(sym_h[k], cdf, sz, offs), range(gn)))
-                    off = np.zeros(gn + 1, dtype=np.int64)
-                    np.cumsum([len(s) for s in streams], out=off[1:])
-                    payload = np.frombuffer(b''.join(streams), dtype=np.uint8)
-                if status is not None:
-                    fe.check_decode_status(status)
-                native_write([paths[k] for k in order[lo:lo + gn]], np.broadcast_to(hdr1, (gn, 16)),
-                             payload, off, self.workers)
+                self._code_and_write(sym_out, [paths[k] for k in order[lo:lo + gn]], st, status)
                 lo += gn
             main.synchronize()
 
+
+    def _code_and_write(self, sym_out, paths, st, status=None):
+        """Entropy-code the symbols ``sym_out`` (n x cb x lh*lw on the device, complete in the
+        current stream's order) of one group and write them as the chunk files ``paths``
+        (.partial, renamed): the device coder from ``GPU_CODER_MIN_STREAMS`` streams up, host
+        coder threads below.  ``status``: the device decoder's status of the group's old chunks,
+        checked before any file is written."""
+        tc, fe, gn = self.tc, self.fact_ent, len(paths)
+        if gn >= fe.GPU_CODER_MIN_STREAMS:
+            packed, off = fe.encode_symbols_device(sym_out)
+            host = tc.pinned('region_write_streams', packed.numel())
+            host.copy_(packed, non_blocking=True)
+            torch.cuda.current_stream(tc.dev).synchronize()
+            payload = host.numpy()
+            st['device_coded'] += gn
+        else:
+            sym_h = sym_out.cpu().numpy()
+            cdf, sz, offs = self._tables
+            streams = list(self._threads().map(
+                lambda k: encode_symbols(sym_h[k], cdf, sz, offs), range(gn)))
+            off = np.zeros(gn + 1, dtype=np.int64)
+            np.cumsum([len(s) for s in streams], out=off[1:])
+            payload = np.frombuffer(b''.join(streams), dtype=np.uint8)
+        if status is not None:
+            fe.check_decode_status(status)
+        hdr1 = np.frombuffer(struct.pack('>QQ', self.ps, self.ps), dtype=np.uint8)
+        native_write(paths, np.broadcast_to(hdr1, (gn, 16)), payload, off, self.workers)
 
 class SlideLevel:
     """The slide at 1/``f`` of its resolution (``CompressedSlide.downsampled(f)``), read-only.
@@ -703,3 +969,41 @@ class SlideLevel:
 
     def __setitem__(self, key, value):
         raise TypeError('a downsampled view is read-only: write to the slide it was taken from')
+
+
+class StoredLevel:
+    """A stored pyramid level (``CompressedSlide.level(k)``), read-only: the ``'cae'`` array
+    ``<group>/k`` that ``build_pyramid`` wrote, read with the slide's model, buffers, lock, pool
+    and ``stats`` (switching levels captures no graphs and loads no model).  Its pixels are the
+    ones a ``CompressedSlide`` opened on ``data_group='<group>/k'`` reads."""
+
+    def __init__(self, slide, k):
+        self._slide = slide
+        self._arr = DirArray(os.path.join(slide._pyramid_group(), str(k)), mode='r')
+        self.downsample = 2 ** k
+        self.shape, self.chunks, self.dtype = self._arr.shape, self._arr.chunks, self._arr.dtype
+        want = level_shape(slide.shape, self.downsample)
+        if ((self._arr.compressor_config or {}).get('id') != 'cae' or self.shape != want
+                or self.chunks != slide.chunks or self.dtype != slide.dtype):
+            raise ValueError('%s is not a level %d of this slide: expected a %r uint8 \'cae\' '
+                             'array in %r chunks' % (self._arr.path, k, want, slide.chunks))
+
+    def read_regions(self, boxes, h, w, out=None):
+        """The ``h`` x ``w`` windows at ``boxes`` of the level; as the slide's ``read_regions``,
+        in level pixels."""
+        yx = np.asarray(boxes, dtype=np.int64).reshape(-1, 2)
+        return self._slide._read(yx, int(h), int(w), out, (len(yx), int(h), int(w), self.shape[2]),
+                                 arr=self._arr)
+
+    def read_region(self, y, x, h, w, out=None):
+        """One ``h`` x ``w`` x c window at (y, x) of the level; ``out`` as for
+        ``read_regions``."""
+        return self._slide._read(np.array([[y, x]], dtype=np.int64), int(h), int(w), out,
+                                 (int(h), int(w), self.shape[2]), arr=self._arr)
+
+    def __getitem__(self, key):
+        """zarr-style basic indexing on Y and X of the level: a host ndarray."""
+        return _getitem(self, key)
+
+    def __setitem__(self, key, value):
+        raise TypeError('a stored level is read-only: write to the slide and rebuild the pyramid')

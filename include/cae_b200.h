@@ -440,6 +440,20 @@ int cae_tiles_crop_reduce_u8(const uint8_t *tiles, int n_tiles, int ps, int c, i
                              int32_t *pieces_dev /*m x 12*/, uint8_t *out, int n_boxes, int box_h,
                              int box_w, void *stream);
 
+/* Resolution pyramid: levels 1..K (1 <= K <= 9, 2^K divides ps) of one batch of decoded tiles in
+ * one launch, each tile read once.  recs[4t .. 4t+3] = {i, j, vh, vw}: tile t is chunk (i, j) of
+ * a gy x gx level-0 chunk grid, with in-array extent 0 < vh, vw <= ps.  `out` holds one chunk row
+ * of every level, level after level: level k is ceil(gx / 2^k) tile-major ps x ps x c tiles,
+ * starting at tile sum_{l<k} ceil(gx / 2^l).  Tile t's level-k pixels (the means of
+ * cae_tiles_crop_reduce_u8 at f = 2^k: rounded half up, over level-0 pixels inside vh x vw only)
+ * go to tile j >> k of level k at rows (i mod 2^k) ps/2^k + [0, ceil(vh/2^k)) and columns
+ * (j mod 2^k) ps/2^k + [0, ceil(vw/2^k)); no other byte of `out` is written.  The tiles of one
+ * call must be distinct chunks of one level-1 chunk row (equal i >> 1).  Checked on the host like cae_tiles_crop_u8; `recs_dev`: DEVICE,
+ * n_tiles x 4 int32, 16-byte aligned.                                                          */
+int cae_tiles_pyramid_u8(const uint8_t *tiles, int n_tiles, int ps, int c, int levels,
+                         const int32_t *recs /*HOST, n_tiles x 4*/, int32_t *recs_dev, int gy,
+                         int gx, uint8_t *out, void *stream);
+
 /* ---- evaluation sums on the device (SURVEY.md 8f-4) ------------------------------------------ */
 /* sse[i] += sum over the per_image uint8 values of image i of (a - b)^2: the numerator of
  * compute_rmse / compute_psnr (src/test_cae.py:57-63, computed there on the host after a full
