@@ -20,6 +20,7 @@ module does the same work B200-first:
 
 Everything here is plumbing around kernels of ``libcae_b200.so``; there is no CPU fallback.
 """
+import contextlib
 import ctypes
 import struct
 import threading
@@ -30,6 +31,7 @@ import torch
 
 from . import _cabi as C
 from . import _ops as O
+from ._entropy import encode_symbols
 from ._store import native_gather, native_read, native_write
 
 
@@ -78,6 +80,14 @@ def _stream_ptr(s):
     return ctypes.c_void_p(s.cuda_stream)
 
 
+@torch.no_grad()
+def encode_tiles(enc, fe, x):
+    """The analysis transform ``enc`` and the quantizer of the entropy bottleneck ``fe`` on uint8
+    tiles N x ps x ps x c (device, current stream) -> int32 symbols N x C x lh x lw."""
+    _, _, sym, _, _ = fe._quantize_cuda(enc(x), want_yq=False, want_p=False, want_sym=True)
+    return sym
+
+
 class TileCodec:
     """The device side for one model and one tile size: ``slots`` input / output buffer slots of
     ``batch`` tiles each, the per-batch kernels captured in CUDA graphs (one per slot)."""
@@ -98,6 +108,8 @@ class TileCodec:
         self.sym_in = [torch.empty((batch, self.cb, self.lh, self.lw), dtype=torch.int32,
                                    device=self.dev) for _ in range(slots)]
         self._enc_g = [None] * slots      # (graph, static symbols out)
+        self.x_level = None               # staging batch of pyramid level tiles (encode_level)
+        self._lvl_g = None                # (graph, static symbols out) of x_level
         self._dec_g = [None] * slots      # (graph, static uint8 out)
         self._keep = []
         self.launches_enc = self.launches_dec = 0
@@ -112,12 +124,9 @@ class TileCodec:
         self._bufs = {}
 
     # ---- the per-batch work, eager form (also what the graphs capture) ----
-    @torch.no_grad()
     def encode_eager(self, x):
         """uint8 N x ps x ps x c (device) -> int32 symbols N x C x lh x lw."""
-        y = self.enc(x)
-        _, _, sym, _, _ = self.fe._quantize_cuda(y, want_yq=False, want_p=False, want_sym=True)
-        return sym
+        return encode_tiles(self.enc, self.fe, x)
 
     @torch.no_grad()
     def decode_eager(self, sym):
@@ -166,6 +175,24 @@ class TileCodec:
             return out
         return self.encode_eager(self.x[slot][:n])
 
+    def encode_level(self, n):
+        """``encode`` of ``self.level_stage()[:n]``, the staging batch of ``region.PyramidWriter``
+        (its own graph: the upload slots belong to the tile loop's upload stream)."""
+        if n == self.batch and self.graphs:
+            if self._lvl_g is None:
+                g, out, _ = self._capture(self.encode_eager, self.level_stage())
+                self._lvl_g = (g, out)
+            g, out = self._lvl_g
+            g.replay()
+            return out
+        return self.encode_eager(self.level_stage()[:n])
+
+    def level_stage(self):
+        if self.x_level is None:
+            self.x_level = torch.empty((self.batch, self.ps, self.ps, self.c_img),
+                                       dtype=torch.uint8, device=self.dev)
+        return self.x_level
+
     def decode(self, slot, n):
         """Run de-quantizer + synthesis transform on ``self.sym_in[slot][:n]``; returns the uint8
         tiles (valid until the slot is decoded again)."""
@@ -195,11 +222,15 @@ class TileCodec:
                                                  pin_memory=True)
         return buf[:nbytes]
 
-    def warm(self, encode=True, decode=True):
-        """Build the graphs of every slot up front (outside any timed region)."""
+    def warm(self, encode=True, decode=True, level=False):
+        """Build the graphs of every slot (and with ``level`` the one of ``encode_level``) up
+        front (outside any timed region)."""
         if not self.graphs:
             return
         built = False
+        if level and self._lvl_g is None:
+            self.encode_level(self.batch)
+            built = True
         for s in range(self.slots):
             if encode and self._enc_g[s] is None:
                 self.encode(s, self.batch)
@@ -283,14 +314,57 @@ def default_schedule(n_tiles, batch, decode=False, cap=8192):
     return group_sizes(n_tiles, sizes + [left - tail, tail], batch)
 
 
+def code_and_write(fe, tables, sym, paths, ps, workers, pinned, pool, status=None,
+                   lock=contextlib.nullcontext()):
+    """Entropy-code the symbols ``sym`` (n x cb x lh*lw on the device, complete in the current
+    stream's order) of one group and write them as the ps^2 chunk files ``paths`` (.partial,
+    renamed): the device coder from ``fe.GPU_CODER_MIN_STREAMS`` streams up (its packed streams
+    come back through the page-locked buffer ``pinned(nbytes)``), host coder threads of ``pool``
+    with the host ``tables`` below.  ``status``: a device decoder status checked before any file
+    is written.  ``lock`` is held around the device coder call and the download of its streams
+    (the device coder calls of one codec share scratch buffers), not around the file writes.
+    Returns (bytes written, streams coded on the device)."""
+    gn = len(paths)
+    device_coded = 0
+    if gn >= fe.GPU_CODER_MIN_STREAMS:
+        with lock:
+            packed, off = fe.encode_symbols_device(sym)
+            host = pinned(packed.numel())
+            host.copy_(packed, non_blocking=True)
+            torch.cuda.current_stream(sym.device).synchronize()
+        payload = host.numpy()
+        device_coded = gn
+    else:
+        sym_h = sym.cpu().numpy()
+        cdf, sz, offs = tables
+        streams = list(pool.map(lambda k: encode_symbols(sym_h[k], cdf, sz, offs), range(gn)))
+        off = np.zeros(gn + 1, dtype=np.int64)
+        np.cumsum([len(s) for s in streams], out=off[1:])
+        payload = np.frombuffer(b''.join(streams), dtype=np.uint8)
+    if status is not None:
+        fe.check_decode_status(status)
+    hdr1 = np.frombuffer(struct.pack('>QQ', ps, ps), dtype=np.uint8)
+    native_write(paths, np.broadcast_to(hdr1, (gn, 16)), payload, off, workers)
+    return int(off[-1]) + 16 * gn, device_coded
+
+
 def compress_tiles(tc, src, tiles, chunk_path, header_hw, workers, coder_tiles, stats,
-                   device_source=None):
+                   device_source=None, level_arrays=None):
     """The 'cae' codec over ``tiles`` (list of (i, j) chunk indices) of the H x W x c uint8 slide
     ``src``: every tile is zero-padded to the full chunk, encoded, and written to
     ``chunk_path((i, j, 0))`` as '>QQ'(h, w) + rANS stream (R:549-555).
 
     ``device_source``: optional uint8 device tensor N x ps x ps x c holding the same tiles in
-    order (inputs already resident in HBM: the device-resident measurement of bench.py)."""
+    order (inputs already resident in HBM: the device-resident measurement of bench.py).
+
+    ``level_arrays``: optional ``DirArray`` of levels 1..K (``tiles`` must then be the whole
+    slide in row-major order, read from ``src``; not with ``device_source``): every uploaded
+    batch is also reduced into the levels (``region.PyramidWriter``) on the main stream after its
+    encode; the level tiles are encoded in whole batches (``encode_level``, main stream) and coded
+    through this call's coder workers.  Adds ``level_chunks`` and ``level_bytes`` to ``stats``."""
+    if level_arrays and device_source is not None:
+        raise ValueError('level_arrays: the levels are reduced from the uploaded source tiles, '
+                         'not from device_source')
     H, W, c = src.shape if src is not None else (0, 0, tc.c_img)
     ps, B, dev = tc.ps, tc.batch, tc.dev
     fe = tc.fe
@@ -317,6 +391,36 @@ def compress_tiles(tc, src, tiles, chunk_path, header_hw, workers, coder_tiles, 
     code_lock = threading.Lock()
     jobs = []
     hdr1 = np.frombuffer(struct.pack('>QQ', *header_hw), dtype=np.uint8)
+    pyr = None
+    if level_arrays:
+        from .region import PyramidWriter
+        level_jobs = []
+        level_lock = threading.Lock()         # one level group at a time: one streams buffer
+        pool = ThreadPoolExecutor(max_workers=workers)       # host coder of small level groups
+        tables = fe._host_tables()
+
+        def code_level(sym, paths, ready):
+            torch.cuda.set_device(dev)
+            # code_lock around the device coder call only (as code_group): level-file writes do
+            # not hold up the next level-0 coder call
+            with level_lock, torch.cuda.stream(s_code):
+                s_code.wait_event(ready)
+                nbytes, _ = code_and_write(fe, tables, sym, paths, ps, workers,
+                                           lambda n: tc.pinned('level_streams', n), pool,
+                                           lock=code_lock)
+                stats.add('level_bytes', nbytes)
+
+        def level_group(sym, paths):
+            ready = torch.cuda.Event()
+            ready.record(main)
+            level_jobs.append(coder.submit(code_level, sym, paths, ready))
+
+        pyr = PyramidWriter((H, W, c), ps, len(level_arrays), B, dev,
+                            lambda k, idx: level_arrays[k - 1].chunk_file(idx),
+                            lambda run: tc.encode_level(len(run)), level_group,
+                            (tc.cb, tc.lh * tc.lw), stage=tc.level_stage())
+        stats['level_chunks'] = len(pyr.paths)
+        stats['level_bytes'] = 0
 
     import time as _t
     t00 = _t.perf_counter()
@@ -386,6 +490,10 @@ def compress_tiles(tc, src, tiles, chunk_path, header_hw, workers, coder_tiles, 
                 ev_up[slot].record(s_in)
             main.wait_event(ev_up[slot])
             sym = tc.encode(slot, n)
+            if pyr is not None:
+                # on the main stream, before ev_free: the next upload into the slot waits for the
+                # reduction; the upload stream waits for nothing else of the levels (DESIGN 3.5f)
+                pyr.add(tc.x[slot], tile_yx[k0:k0 + n])
             ev_free[slot] = torch.cuda.Event()
             ev_free[slot].record(main)
         if gpos == 0 and coded[gi] is not None:
@@ -406,10 +514,14 @@ def compress_tiles(tc, src, tiles, chunk_path, header_hw, workers, coder_tiles, 
             glo += gpos
             gpos = 0
             gi = (gi + 1) % len(sym_all)
+    if pyr is not None:
+        pyr.finish()
     mark('c_all_batches_issued')
-    for j in jobs:
+    for j in jobs + (level_jobs if pyr is not None else []):
         j.result()
     coder.shutdown()
+    if pyr is not None:
+        pool.shutdown()
     for st in (main, s_in, s_code):        # this call's streams only: another call may be in flight
         st.synchronize()
     mark('c_done')

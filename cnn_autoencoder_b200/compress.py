@@ -28,6 +28,7 @@ import torch
 from . import _autoencoders as AE
 from ._entropy import encode_symbols
 from . import _slide
+from . import region
 from ._store import DirArray, can_native_gather, native_gather, native_write, padded_tile
 
 _models = {}
@@ -150,14 +151,54 @@ def as_yxc(src, data_axes):
     return _AxesView(src, axes)
 
 
+def check_levels(levels, shape, ps, save_as_bottleneck=False, world_size=1, data_group='0/0'):
+    """The number K of pyramid levels ``compress_image(..., levels=levels)`` writes for a
+    Y x X x c source in ps^2 chunks (0: none).  ``levels``: 0, K >= 1 (``region.check_levels``) or
+    ``'auto'`` (``region.default_levels``).  Raises ``ValueError`` for a bad K, and for levels with
+    ``save_as_bottleneck``, ``world_size > 1`` or a data group whose last component is not ``0``."""
+    if isinstance(levels, str):
+        if levels != 'auto':
+            raise ValueError("levels must be an int or 'auto', got %r" % (levels,))
+        K = region.default_levels(shape, ps)
+    elif isinstance(levels, (int, np.integer)) and not isinstance(levels, (bool, np.bool_)) \
+            and int(levels) == 0:
+        return 0
+    else:
+        K = region.check_levels(levels, ps)
+    if save_as_bottleneck:
+        raise ValueError('levels: a latent store (save_as_bottleneck) has no pixel levels')
+    if world_size > 1:
+        raise ValueError('levels: the shards of a sharded job are contiguous tile ranges that split '
+                         'chunk rows; compress without levels, then run '
+                         "CompressedSlide(path, checkpoint, mode='r+').build_pyramid()")
+    if region.pyramid_group('', data_group) is None:
+        raise ValueError("levels go beside a '<group>/0' array; the data group is %r" % (data_group,))
+    return K
+
+
 def compress_image(codec, checkpoint, input_filename, output_filename, patch_size=512,
                    source_format='zarr', data_group='0/0', data_axes='TCZYX',
                    progress_bar=False, save_as_bottleneck=False, gpu=False, *,
-                   rank=None, world_size=None, batch_tiles=16, workers=None, coder_tiles=None):
+                   rank=None, world_size=None, batch_tiles=16, workers=None, coder_tiles=None,
+                   levels=0):
     """Same positional signature as the reference (``compress.py:29-36``); the keyword-only
     arguments select this process's shard, the GPU batch size and how many tiles are entropy
     coded per device call (one size, or a schedule of group sizes: ``_slide.group_sizes``).  Returns a dict of counters (tiles, pixels, bytes, seconds,
-    device_coded) for the caller's throughput report."""
+    device_coded) for the caller's throughput report.
+
+    ``levels``: also write the resolution pyramid in the same pass (0: no, the default; K: levels
+    1..K; ``'auto'``: ``region.default_levels``; see ``check_levels``).  Level k is the ``'cae'``
+    array ``<group>/k`` beside ``<group>/0``, with the same codec config and chunks; its files are
+    the ones this function writes for ``reduce(source, 2^k)``, the block means of the *source*
+    rounded half up (edge blocks average the pixels inside the array), and ``<group>/.zattrs``
+    gets the ``multiscales`` entry of ``CompressedSlide.build_pyramid``.  This is the one
+    difference from ``build_pyramid``, whose levels are means of the decoded slide: levels
+    written here carry one lossy encode, not two.  Every uploaded batch is reduced into one
+    chunk row per level on the device (``region.PyramidWriter``); nothing is decoded.  An
+    existing entry is removed before any chunk is written and the new one is written last, so a
+    failed call leaves no entry listing incomplete levels; the chunks of levels 1..K are removed
+    like level 0's, and stored levels above K are left in place, unlisted.  The stats gain
+    ``level_chunks`` and ``level_bytes``; ``bytes``, ``tiles`` and ``pixels`` count level 0."""
     if 'CAE' not in codec:
         raise ValueError('Codec %s not supported' % codec)
     if not torch.cuda.is_available():
@@ -167,6 +208,7 @@ def compress_image(codec, checkpoint, input_filename, output_filename, patch_siz
     src = as_yxc(open_source(input_filename, data_group), data_axes)
     H, W, C = src.shape
     ps = patch_size
+    K = check_levels(levels, (H, W, C), ps, save_as_bottleneck, world_size, data_group)
 
     model = load_model(checkpoint)
     fact_ent = model['fact_ent'].module
@@ -196,6 +238,11 @@ def compress_image(codec, checkpoint, input_filename, output_filename, patch_siz
         comp = _CodecConfig('cae', checkpoint=checkpoint if isinstance(checkpoint, str) else '<dict>',
                             gpu=gpu)
         meta = dict(shape=(H, W, C), chunks=(ps, ps, C), dtype=np.uint8)
+    level_arrays = []
+    if K:
+        group = region.pyramid_group(output_filename, data_group)
+        if 'multiscales' in region._read_attrs(group):
+            region.write_multiscales(output_filename, group, 0)
     if rank == 0:
         dst = DirArray(out_path, compressor=comp, mode='w', **meta)
         if world_size == 1:
@@ -203,6 +250,11 @@ def compress_image(codec, checkpoint, input_filename, output_filename, patch_siz
             # array that was there before are gone.  The ranks of a sharded job have no barrier
             # between this and the first chunk another rank writes, so there stale chunks stay.
             dst.remove_chunks(workers)
+        for k in range(1, K + 1):
+            level_arrays.append(DirArray(os.path.join(group, str(k)), compressor=comp, mode='w',
+                                         shape=region.level_shape((H, W, C), 2 ** k),
+                                         chunks=(ps, ps, C), dtype=np.uint8))
+            level_arrays[-1].remove_chunks(workers)
     else:
         while not os.path.exists(os.path.join(out_path, '.zarray')):
             time.sleep(0.05)
@@ -221,13 +273,16 @@ def compress_image(codec, checkpoint, input_filename, output_filename, patch_siz
         # streams of a group coded on the device (see _slide.py)
         tc = _slide.tile_codec(model, ps, C, batch_tiles)
         if len(mine) >= batch_tiles:
-            tc.warm(encode=True, decode=False)
+            tc.warm(encode=True, decode=False, level=bool(K))
         t_start = time.perf_counter()
         st = _slide._Stats(want_trace=bool(os.environ.get('CAE_SLIDE_TRACE')))
-        _slide.compress_tiles(tc, src, mine, dst.chunk_file, (ps, ps), workers, coder_tiles, st)
+        _slide.compress_tiles(tc, src, mine, dst.chunk_file, (ps, ps), workers, coder_tiles, st,
+                              level_arrays=level_arrays)
         stats.update(st)
         stats['engine'] = 'slide'
         stats['seconds'] = time.perf_counter() - t_start
+        if K:
+            region.write_multiscales(output_filename, group, K)
         return stats
     if not isinstance(coder_tiles, (int, np.integer)):
         coder_tiles = max(int(g) for g in coder_tiles)     # a group schedule (_slide.group_sizes)
@@ -238,6 +293,13 @@ def compress_image(codec, checkpoint, input_filename, output_filename, patch_siz
     coder_stream = torch.cuda.Stream()             # of the next group run on the main stream
     coder_jobs = []
     out_pin = [None]                               # reused pinned buffer of the coder thread
+
+    def coder_pinned(n):
+        # page-locked allocations stall every other CUDA call of the process: one buffer for
+        # every group of the coder thread, only grown
+        if out_pin[0] is None or out_pin[0].numel() < n:
+            out_pin[0] = torch.empty(int(n * 1.25) + 4096, dtype=torch.uint8, pin_memory=True)
+        return out_pin[0][:n]
     device = torch.cuda.current_device()
 
     def write_stream(idx, h, w, data):
@@ -264,12 +326,7 @@ def compress_image(codec, checkpoint, input_filename, output_filename, patch_siz
                 with torch.cuda.stream(coder_stream):
                     coder_stream.wait_event(ready)
                     packed, off = fact_ent.encode_symbols_device(sym)
-                    # page-locked allocations stall every other CUDA call of the process: keep
-                    # one buffer for all groups and only grow it
-                    if out_pin[0] is None or out_pin[0].numel() < packed.numel():
-                        out_pin[0] = torch.empty(int(packed.numel() * 1.25) + 4096,
-                                                 dtype=torch.uint8, pin_memory=True)
-                    host = out_pin[0][:packed.numel()]
+                    host = coder_pinned(packed.numel())
                     host.copy_(packed, non_blocking=True)
                     coder_stream.synchronize()
                 # one native call writes the group's chunk files (16-byte header + stream each)
@@ -336,6 +393,8 @@ def compress_image(codec, checkpoint, input_filename, output_filename, patch_siz
         lh, lw = y.shape[2], y.shape[3]
         hh, ww = (lh, lw) if save_as_bottleneck else (th, tw)
         stats['pixels'] += len(batch) * th * tw
+        if pyr is not None:
+            pyr.add(x, [ij for ij, _ in batch])
         g = acc.setdefault((lh, lw), dict(sym=[], meta=[]))
         g['sym'].append(sym)
         g['meta'] += [((idx[0], idx[1], 0), hh, ww) for idx, _ in batch]
@@ -364,6 +423,30 @@ def compress_image(codec, checkpoint, input_filename, output_filename, patch_siz
         ring.append(ring.pop(0))
         return ring[-1]
 
+    pyr = None
+    if K:
+        def level_group(sym, paths):
+            ready = torch.cuda.Event()
+            ready.record()
+
+            def job():
+                # through the coder thread, which serialises the device coder calls
+                torch.cuda.set_device(device)
+                with torch.cuda.stream(coder_stream):
+                    coder_stream.wait_event(ready)
+                    nbytes, _ = _slide.code_and_write(fact_ent, (cdf, sizes, offs), sym, paths, ps,
+                                                      workers, coder_pinned, pool)
+                stats['level_bytes'] += nbytes
+                return []
+            coder_jobs.append(coder.submit(job))
+
+        # chunks come in row-major order: the batches are reduced as they are encoded
+        pyr = region.PyramidWriter((H, W, C), ps, K, batch_tiles, device,
+                                   lambda k, idx: level_arrays[k - 1].chunk_file(idx),
+                                   lambda run: _slide.encode_tiles(model['encoder'], fact_ent, run),
+                                   level_group, (channels_bn, (ps // 2 ** level) ** 2))
+        stats.update(level_chunks=len(pyr.paths), level_bytes=0)
+
     groups = {}
     for k0 in range(0, len(mine), batch_tiles):
         part = mine[k0:k0 + batch_tiles]
@@ -384,6 +467,8 @@ def compress_image(codec, checkpoint, input_filename, output_filename, patch_siz
             run_batch(g)
     for key in list(acc):
         flush_group(key, final=True)
+    if pyr is not None:
+        pyr.finish()
     t0 = time.perf_counter()
     for j in coder_jobs:
         writes += j.result()
@@ -393,6 +478,8 @@ def compress_image(codec, checkpoint, input_filename, output_filename, patch_siz
     coder.shutdown()
     pool.shutdown()
     torch.cuda.synchronize()
+    if K:
+        region.write_multiscales(output_filename, group, K)
     stats['seconds'] = time.perf_counter() - t_start
     return stats
 
@@ -420,7 +507,7 @@ def compress(args):
         st = compress_image(codec=args.codec, checkpoint=args.checkpoint, input_filename=fn,
                             output_filename=out, patch_size=args.patch_size,
                             data_group=args.data_group, save_as_bottleneck=args.save_as_bottleneck,
-                            gpu=True, batch_tiles=args.batch_tiles)
+                            gpu=True, batch_tiles=args.batch_tiles, levels=args.levels)
         print('Compressed image %s into %s: %d tiles, %.1f MP/s' % (
             fn, out, st['tiles'], st['pixels'] / 1e6 / max(st['seconds'], 1e-9)))
 
@@ -436,7 +523,18 @@ def _parser():
     ap.add_argument('-sbn', '--save-as-bottleneck', action='store_true')
     ap.add_argument('-g', '--gpu', action='store_true')
     ap.add_argument('--batch-tiles', type=int, default=16)
+    ap.add_argument('--levels', type=_levels_arg, default=0,
+                    help="also write pyramid levels 1..K (an int, or 'auto'); off by default")
     return ap
+
+
+def _levels_arg(text):
+    if text == 'auto':
+        return text
+    try:
+        return int(text)
+    except ValueError:
+        raise argparse.ArgumentTypeError("expected an int or 'auto', got %r" % text) from None
 
 
 if __name__ == '__main__':

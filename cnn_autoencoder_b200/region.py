@@ -37,8 +37,8 @@ import torch
 from . import _autoencoders as AE
 from . import _cabi as C
 from . import _slide
-from ._entropy import decode_symbols, encode_symbols
-from ._store import DirArray, _paths_blob, native_read, native_write
+from ._entropy import decode_symbols
+from ._store import DirArray, _paths_blob, native_read
 
 
 def plan(shape, chunks, boxes, box_h, box_w):
@@ -247,6 +247,118 @@ def pyramid_place(shape, ps, k, chunk_yx):
     return np.stack([j >> k, (i % f) * lps, (j % f) * lps, -(-vh // f), -(-vw // f)], 1)
 
 
+def pyramid_group(store, data_group):
+    """The directory that holds the levels of the array ``<store>/<data_group>`` (``<group>`` of a
+    ``<group>/0`` data group), or None when the data group's last component is not ``0``."""
+    parts = [p for p in (data_group or '').split('/') if p]
+    if not parts or parts[-1] != '0':
+        return None
+    return os.path.join(store, *parts[:-1])
+
+
+class PyramidWriter:
+    """Levels 1..K of a Y x X x c slide in ps^2 chunks whose level-0 tiles arrive in row-major
+    order, batch by batch (``add``), each written as soon as it is complete.
+
+    After each batch, ``cae_tiles_pyramid_u8`` reduces the batch's tiles into one chunk-row buffer
+    per level (one launch per level-0 chunk row of the batch, so that rows of different level-1
+    chunk rows never share the buffer).  Once the last level-0 row of a level chunk row has been
+    reduced (``pyramid_rows`` order), its tiles are copied into a staging batch, which goes to
+    ``encode(run)`` (a device uint8 run of ``batch`` tiles, fewer only at the end of a group -> its
+    int32 symbols, in the current stream's order) whenever it is full: whole batches keep the
+    encoder's buffers at one size.  The symbols are collected into coder groups
+    (``_slide.group_sizes`` of the default schedule); each full group goes to
+    ``code_and_write(sym, paths)`` with the chunk files ``level_path(k, (R, col, 0))`` of its
+    tiles.  Beyond the caller's own memory this holds one chunk row per level, one batch of tiles
+    and one group of symbols.  Everything runs on the current stream.  ``stage``: the device
+    buffer of ``batch`` tiles to use as the staging batch (default a new one), so that a caller
+    can replay a graph captured on it."""
+
+    def __init__(self, shape, ps, levels, batch, device, level_path, encode, code_and_write,
+                 sym_shape, stage=None):
+        from ._slide import default_schedule, group_sizes
+        self.shape, self.ps, self.levels, self.batch = tuple(shape), ps, levels, batch
+        self.dev = device
+        self.encode, self.code_and_write, self.sym_shape = encode, code_and_write, tuple(sym_shape)
+        self.gy, self.gx = -(-int(shape[0]) // ps), -(-int(shape[1]) // ps)
+        self.widths = [-(-self.gx // 2 ** k) for k in range(1, levels + 1)]
+        self.first = np.concatenate([[0], np.cumsum(self.widths)]).astype(int)
+        # one chunk row per level, back to back: the layout cae_tiles_pyramid_u8 writes
+        self.rows = torch.zeros((int(self.first[-1]), ps, ps, int(shape[2])), dtype=torch.uint8,
+                                device=device)
+        self.order = pyramid_rows(self.gy, levels)
+        self.paths = [level_path(k, (R, col, 0)) for k, R in self.order
+                      for col in range(self.widths[k - 1])]
+        self._groups = iter(group_sizes(len(self.paths), default_schedule(len(self.paths), batch),
+                                        batch))
+        self._gn, self._g0, self._lo, self._sym = next(self._groups), 0, 0, None
+        self._x = stage if stage is not None else torch.empty(
+            (batch, ps, ps, int(shape[2])), dtype=torch.uint8, device=device)
+        self._fill = 0                  # tiles in the staging batch
+        self._done = 0                  # level-0 chunk rows reduced so far
+        self.flushed = []               # the level chunk rows handed to the encoder, in order
+        self._recs_dev = torch.empty(4 * batch, dtype=torch.int32, device=device)
+
+    def add(self, tiles, chunk_yx):
+        """Reduce a batch: ``tiles`` (n x ps x ps x c uint8 on the device, contiguous) are the
+        level-0 chunks ``chunk_yx`` (n x 2, row-major, after every chunk of earlier batches)."""
+        ij = np.asarray(chunk_yx, dtype=np.int64).reshape(-1, 2)
+        cuts = np.flatnonzero(np.diff(ij[:, 0])) + 1
+        for a, b in zip(np.concatenate([[0], cuts]), np.concatenate([cuts, [len(ij)]])):
+            self.complete(int(ij[a, 0]))         # the rows before this one are reduced
+            self._launch(tiles, int(a), int(b), ij)
+
+    def finish(self):
+        """Write what is left once every level-0 chunk has been added."""
+        self.complete(self.gy)
+
+    def complete(self, upto):
+        """Flush every level chunk row whose last level-0 row is below ``upto``."""
+        for i in range(self._done, upto):
+            for k in range(1, self.levels + 1):
+                if (i + 1) % 2 ** k == 0 or i == self.gy - 1:
+                    self._flush(k, i >> k)
+        self._done = max(self._done, upto)
+
+    def _launch(self, tiles, a, b, ij):
+        ps, c = self.ps, int(self.shape[2])
+        vh = np.minimum(ps, self.shape[0] - ij[a:b, 0] * ps)
+        vw = np.minimum(ps, self.shape[1] - ij[a:b, 1] * ps)
+        recs = np.ascontiguousarray(np.stack([ij[a:b, 0], ij[a:b, 1], vh, vw], 1), dtype=np.int32)
+        C.check(C.lib().cae_tiles_pyramid_u8(
+            tiles.data_ptr() + a * ps * ps * c, b - a, ps, c, self.levels, recs.ctypes.data,
+            self._recs_dev.data_ptr(), self.gy, self.gx, self.rows.data_ptr(),
+            _slide._stream_ptr(torch.cuda.current_stream(self.dev))))
+
+    def _encode(self):
+        n = self._fill
+        if self._sym is None:
+            self._sym = torch.empty((self._gn,) + self.sym_shape, dtype=torch.int32, device=self.dev)
+        self._sym[self._g0:self._g0 + n].copy_(self.encode(self._x[:n]).reshape((n,) + self.sym_shape),
+                                               non_blocking=True)
+        self._g0 += n
+        self._fill = 0
+        if self._g0 == self._gn:
+            self.code_and_write(self._sym, self.paths[self._lo:self._lo + self._gn])
+            self._lo += self._gn
+            self._gn, self._g0, self._sym = next(self._groups, 0), 0, None
+
+    def _flush(self, k, R):
+        """Encode level k's finished chunk row R, code every group it fills, clear the row."""
+        row = self.rows[self.first[k - 1]:self.first[k]]
+        a = 0
+        while a < len(row):
+            f = self._fill
+            m = min(len(row) - a, self.batch - f, self._gn - self._g0 - f)
+            self._x[f:f + m].copy_(row[a:a + m], non_blocking=True)
+            self._fill += m
+            a += m
+            if self._fill == self.batch or self._g0 + self._fill == self._gn:
+                self._encode()
+        row.zero_()
+        self.flushed.append((k, R))
+
+
 def multiscales(levels, name=''):
     """The OME-Zarr 0.4 style ``multiscales`` entry of levels 0..K (axes y, x, c)."""
     return [{'version': '0.4', 'name': name,
@@ -426,12 +538,8 @@ class CompressedSlide:
         return self if int(k) == 0 else StoredLevel(self, int(k))
 
     def _pyramid_group(self):
-        """The directory holding the levels (``<group>`` of a ``<group>/0`` data group), or None
-        when the data group's last component is not ``0``."""
-        parts = [p for p in (self._data_group or '').split('/') if p]
-        if not parts or parts[-1] != '0':
-            return None
-        return os.path.join(self._store, *parts[:-1])
+        """The directory holding the levels (``pyramid_group``), or None."""
+        return pyramid_group(self._store, self._data_group)
 
     def build_pyramid(self, levels=None, overwrite=False):
         """Write the resolution pyramid: level k = 1..K as a ``'cae'`` array ``<group>/k`` beside
@@ -481,6 +589,7 @@ class CompressedSlide:
         Y, X = self.shape[:2]
         gy, gx = self._arr.grid[:2]
         with self._lock, torch.cuda.device(dev):
+            tc.warm(encode=False, decode=False, level=True)     # before the decode is in flight
             if overwrite:
                 if 'multiscales' in _read_attrs(group):
                     write_multiscales(self._store, group, 0)
@@ -494,72 +603,17 @@ class CompressedSlide:
                     for k, q in zip(range(1, K + 1), level_paths)}
             for a in arrs.values():
                 a.remove_chunks(self.workers)
-            # one chunk row per level, back to back: the layout cae_tiles_pyramid_u8 writes
-            widths = [-(-gx // 2 ** k) for k in range(1, K + 1)]
-            first = np.concatenate([[0], np.cumsum(widths)])
-            rows = torch.zeros((int(first[-1]), ps, ps, c), dtype=torch.uint8, device=dev)
-            order = pyramid_rows(gy, K)
-            paths = [arrs[k].chunk_file((R, col, 0)) for k, R in order
-                     for col in range(widths[k - 1])]
-            groups = iter(_slide.group_sizes(len(paths), _slide.default_schedule(len(paths), B),
-                                             B))
-            st = dict(level_chunks=len(paths), device_coded=0)
-            enc = dict(slot=0, fill=0, lo=0, gn=next(groups), g0=0, sym=None)
-
-            def encode_slot():
-                e = enc
-                n = e['fill']
-                e['sym'][e['g0']:e['g0'] + n].copy_(tc.encode(e['slot'], n).reshape(n, tc.cb, -1),
-                                                    non_blocking=True)
-                e['g0'] += n
-                e['slot'], e['fill'] = (e['slot'] + 1) % tc.slots, 0
-                if e['g0'] == e['gn']:
-                    self._code_and_write(e['sym'], paths[e['lo']:e['lo'] + e['gn']], st)
-                    e['lo'] += e['gn']
-                    e['gn'], e['g0'], e['sym'] = next(groups, 0), 0, None
-
-            def flush(k):
-                """Hand level k's finished chunk row to the encoder and clear it."""
-                row = rows[first[k - 1]:first[k]]
-                a = 0
-                while a < len(row):
-                    e = enc
-                    if e['sym'] is None:
-                        e['sym'] = torch.empty((e['gn'], tc.cb, tc.lh * tc.lw), dtype=torch.int32,
-                                               device=dev)
-                    m = min(len(row) - a, B - e['fill'], e['gn'] - e['g0'] - e['fill'])
-                    tc.x[e['slot']][e['fill']:e['fill'] + m].copy_(row[a:a + m], non_blocking=True)
-                    e['fill'] += m
-                    a += m
-                    if e['fill'] == B or e['g0'] + e['fill'] == e['gn']:
-                        encode_slot()
-                row.zero_()
-
-            done = [0]                   # level-0 chunk rows reduced so far
-
-            def complete(upto):
-                for i in range(done[0], upto):
-                    for k in range(1, K + 1):
-                        if (i + 1) % 2 ** k == 0 or i == gy - 1:
-                            flush(k)
-                done[0] = max(done[0], upto)
-
-            tile_bytes = ps * ps * c
+            st = dict(device_coded=0)
+            pyr = PyramidWriter(self.shape, ps, K, B, dev, lambda k, idx: arrs[k].chunk_file(idx),
+                                lambda run: tc.encode_level(len(run)),
+                                lambda sym, paths: self._code_and_write(sym, paths, st),
+                                (tc.cb, tc.lh * tc.lw), stage=tc.level_stage())
+            st['level_chunks'] = len(pyr.paths)
 
             def step(tiles, n_tiles, part):
                 if tiles is None:        # missing chunks: their level pixels are the zeros rows holds
                     return
-                # one launch per level-0 chunk row of the batch: the rows before it are complete
-                # (chunks come in row-major order) and leave the buffers before its tiles land
-                cuts = np.flatnonzero(np.diff(part[:, 1])) + 1
-                for a, b in zip(np.concatenate([[0], cuts]), np.concatenate([cuts, [n_tiles]])):
-                    complete(int(part[a, 1]))
-                    recs = self._table(part[a:b, 1:5])
-                    C.check(C.lib().cae_tiles_pyramid_u8(
-                        tiles.data_ptr() + int(a) * tile_bytes, int(b - a), ps, c, K,
-                        recs.ctypes.data, self._pieces_dev.data_ptr(), gy, gx, rows.data_ptr(),
-                        _slide._stream_ptr(torch.cuda.current_stream(dev))))
-                complete(int(part[-1, 1]) + (int(part[-1, 2]) == gx - 1))
+                pyr.add(tiles, part[:, 1:3])
 
             ii, jj = np.meshgrid(np.arange(gy), np.arange(gx), indexing='ij')
             chunk_yx = np.stack([ii.ravel(), jj.ravel()], 1)
@@ -567,7 +621,7 @@ class CompressedSlide:
                                np.minimum(ps, Y - chunk_yx[:, 0] * ps),
                                np.minimum(ps, X - chunk_yx[:, 1] * ps)], 1).astype(np.int32)
             self._decode_and_crop(chunk_yx, pieces, step)
-            complete(gy)
+            pyr.finish()
             torch.cuda.current_stream(dev).synchronize()
             self.stats.update(st)
             write_multiscales(self._store, group, K)
@@ -909,26 +963,10 @@ class CompressedSlide:
         (.partial, renamed): the device coder from ``GPU_CODER_MIN_STREAMS`` streams up, host
         coder threads below.  ``status``: the device decoder's status of the group's old chunks,
         checked before any file is written."""
-        tc, fe, gn = self.tc, self.fact_ent, len(paths)
-        if gn >= fe.GPU_CODER_MIN_STREAMS:
-            packed, off = fe.encode_symbols_device(sym_out)
-            host = tc.pinned('region_write_streams', packed.numel())
-            host.copy_(packed, non_blocking=True)
-            torch.cuda.current_stream(tc.dev).synchronize()
-            payload = host.numpy()
-            st['device_coded'] += gn
-        else:
-            sym_h = sym_out.cpu().numpy()
-            cdf, sz, offs = self._tables
-            streams = list(self._threads().map(
-                lambda k: encode_symbols(sym_h[k], cdf, sz, offs), range(gn)))
-            off = np.zeros(gn + 1, dtype=np.int64)
-            np.cumsum([len(s) for s in streams], out=off[1:])
-            payload = np.frombuffer(b''.join(streams), dtype=np.uint8)
-        if status is not None:
-            fe.check_decode_status(status)
-        hdr1 = np.frombuffer(struct.pack('>QQ', self.ps, self.ps), dtype=np.uint8)
-        native_write(paths, np.broadcast_to(hdr1, (gn, 16)), payload, off, self.workers)
+        _, device_coded = _slide.code_and_write(
+            self.fact_ent, self._tables, sym_out, paths, self.ps, self.workers,
+            lambda n: self.tc.pinned('region_write_streams', n), self._threads(), status)
+        st['device_coded'] += device_coded
 
 class SlideLevel:
     """The slide at 1/``f`` of its resolution (``CompressedSlide.downsampled(f)``), read-only.
